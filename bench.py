@@ -22,6 +22,7 @@ seeded layouts).  Prints ONE JSON line (rank 0).  See DESIGN.md "Measurement" fo
   fomaml     config 4: seconds per FOMAML meta-iteration, 32 tasks x (256 support + 256 query) steps, tasks sharded
              over the N GPUs (strong scaling) and 32 tasks PER GPU (weak scaling); one gradient all-reduce per iteration
   --impl reference : only the CPU path, same metric/config, all host cores
+  --dump-outputs DIR : after the timed steps, write what the last one returned to DIR/<name>.npy (see dump_outputs)
 """
 from __future__ import annotations
 
@@ -63,7 +64,14 @@ def parse_args():
     ap.add_argument("--fomaml-iters", type=int, default=5, help="timed FOMAML meta-iterations (after two warm-up ones)")
     ap.add_argument("--fomaml-tasks", type=int, default=32, help="tasks per meta-batch (config 4)")
     ap.add_argument("--fomaml-k", type=int, default=256, help="support and query steps per task (config 4)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the last timed step's outputs (rank 0) as DIR/<name>.npy, to compare two builds")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the GPU path's outputs: not with --impl reference")
+    return args
 
 
 # ----------------------------------------------------------------------------------------- clocks
@@ -313,6 +321,38 @@ def ncu_traffic(envs, kernel=None):
     return None
 
 
+DUMP_ENVS = 1 << 20     # per-env outputs of at most this many envs: 7 float32 arrays (29.4 MB) + a float64 index (8.4 MB)
+DUMP_OBS_ENVS = 512     # observation frames of this many envs: 512 x 56 x 56 x 3 float32 = 19.3 MB
+
+
+def dump_outputs(out_dir, step_out):
+    """Write what one `env.step` returned -- the gymnasium 5-tuple and the info tensors -- to out_dir/<name>.npy as float32,
+    57.1 MB at most.  Per-env outputs are written for every env up to DUMP_ENVS envs, observation frames for DUMP_OBS_ENVS
+    envs; larger batches are sampled with a fixed seed, and the sampled env indices are written as env_index.npy and
+    obs_env_index.npy (float64).  With the same arguments two runs step the same envs with the same actions, so the files
+    of two builds can be compared array for array."""
+    import numpy as np
+    import torch
+    obs, reward, terminated, truncated, info = step_out
+    n = reward.numel()
+    rng = np.random.default_rng(20240611)
+
+    def sample(k):
+        return np.arange(n) if n <= k else np.sort(rng.choice(n, k, replace=False))
+
+    env_index, obs_index = sample(DUMP_ENVS), sample(DUMP_OBS_ENVS)
+    rows = torch.as_tensor(env_index, device=reward.device)
+    arrays = {"env_index": env_index.astype(np.float64), "obs_env_index": obs_index.astype(np.float64),
+              "obs": obs[torch.as_tensor(obs_index, device=obs.device)].float().cpu().numpy()}
+    for name, t in (("reward", reward), ("terminated", terminated), ("truncated", truncated),
+                    ("episode_return", info["episode_return"]), ("episode_length", info["episode_length"]),
+                    ("stuck", info["stuck"]), ("done", info["done"])):
+        arrays[name] = t[rows].float().cpu().numpy()
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 def bench_ppo(args, dev, rank, world, cells, agent, sampler, barrier):
     """End-to-end PPO env-steps/s in the config-3 regime on every GPU (weak scaling: the per-GPU batch is fixed), the
     reference's loop (ppo/ppo_train.py:145-190: collect -> update) and hyper-parameters (lr 3e-4, gamma .99, lambda
@@ -493,13 +533,16 @@ def run_ours(args):
     sampler.mark("timed_start")
     e0.record()
     for i in range(K):
-        env.step(acts[i % ring])
+        last = env.step(acts[i % ring])
     e1.record()
     barrier()
     sampler.mark("timed_end")
     ms = e0.elapsed_time(e1)
     launches = env.launch_count() - launches0
     restarted = int((env.state_numpy()["layout"] != lay0).sum())  # envs that auto-reset onto another layout while timed
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, last)  # before the e2e steps below overwrite the env's output buffers
+    del last
 
     # ---- e2e: host action buffers -> step -> host reward/flags (observations stay in HBM) -------------------
     e2e = None

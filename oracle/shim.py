@@ -7,8 +7,7 @@ modules under /root/reference be imported in this container, where `minigrid` an
 `import src.custom_envs.register`, `src.scenario_creator.scenario_creator.ScenarioCreator`,
 `src.wrappers.*`, `src.ppo.PPO`, `src.fomaml.FOMAML` execute the reference's own code.
 
-Used only by `tests/golden/make_golden.py` (fixture generation) and by the optional
-`tests/test_reference_over_shim.py` (skipped when /root/reference is absent, e.g. on the GPU box).
+Used only by `tests/golden/make_golden.py` (fixture generation); the tests read the fixtures it wrote.
 """
 from __future__ import annotations
 

@@ -55,3 +55,29 @@ def test_bench_tool_small_batch():
         assert key in out, key
     assert out["gpu_launches"] == 16 and out["roofline"]["bound"] == "hbm" and out["e2e"]["h2d_bytes_per_step"] == 32768 * 8
     assert "sym" in out["symbolic_only"]["kernel"] and out["symbolic_only"]["value_per_gpu"] > out["value"]
+
+
+def test_bench_dump_outputs_repeat_exactly(tmp_path):
+    """--dump-outputs: the last timed step's outputs as float .npy files, identical for two runs with the same arguments."""
+    import numpy as np
+    names = {"obs", "obs_env_index", "env_index", "reward", "terminated", "truncated", "episode_return", "episode_length",
+             "stuck", "done"}
+    N, K = 4096, 37
+    dumps = []
+    for run in range(2):
+        d = tmp_path / f"run{run}"
+        lines = _run(["bench.py", "--envs", str(N), "--steps", str(K), "--warmup", "3", "--layouts", "256", "--skip-cpu-baseline",
+                      "--skip-e2e", "--skip-learners", "--dump-outputs", str(d)])
+        out = json.loads(lines[-1])
+        assert out["steps"] == K and out["gpu_launches"] == K
+        assert {p.name for p in d.iterdir()} == {n + ".npy" for n in names}
+        dumps.append({n: np.load(d / (n + ".npy")) for n in names})
+        assert sum(p.stat().st_size for p in d.iterdir()) <= 64 << 20
+    a, b = dumps
+    for n in names:
+        assert a[n].dtype in (np.float32, np.float64), n
+        assert np.array_equal(a[n], b[n]), n
+    assert a["obs"].shape == (512, 56, 56, 3) and a["reward"].shape == (N,)
+    assert np.array_equal(a["env_index"], np.arange(N)) and np.all(np.diff(a["obs_env_index"]) > 0)
+    assert np.array_equal(a["done"], np.maximum(a["terminated"], a["truncated"]))
+    assert np.all((a["episode_length"] > 0) == (a["done"] > 0))
