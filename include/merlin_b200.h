@@ -185,7 +185,9 @@ int merlin_env_rearm(merlin_env_t* h, void* stream);
  * agent_pov=True), src/scenario_creator/scenario_creator.py:48) as a batch op with an optional row gather, so a
  * rollout can keep the 147-byte symbolic image per step and expand minibatches on read (the reference's RolloutBuffer
  * keeps 37 632 B of float32 per step, src/rollout_buffer.py:5).  obs_sym: DEVICE u8[n_rows][7][7][3] as step()/reset()
- * write them; index: DEVICE i64[m] row numbers or NULL (= rows 0..m-1); out: DEVICE u8[m][9408].
+ * write them -- any image Grid.encode can produce renders correctly, also one stepped under an earlier layout pool or
+ * showing objects the current pool does not hold; index: DEVICE i64[m] row numbers or NULL (= rows 0..m-1), a row
+ * outside [0, n_rows) renders row 0; out: DEVICE u8[m][9408].
  * blocked = 0: u8[m][56][56][3], identical to the obs_rgb of step();  blocked = 1: u8[m][14][14][48], every 4x4 pixel
  * block contiguous with channel index c*16 + dy*4 + dx (space-to-depth; what the actor-critic's first layer reads). */
 int merlin_env_render(merlin_env_t* h, const uint8_t* obs_sym, int64_t n_rows, const int64_t* index, int32_t m,

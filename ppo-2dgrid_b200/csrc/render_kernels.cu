@@ -12,6 +12,27 @@ namespace merlin {
 // ---------------------------------------------------------------------------------------------------
 // render_kernel<BLOCKED>: frames from stored symbolic observations, one warp per frame, optional row gather.
 // Rollouts can then keep 147 B per step instead of 9408 B and expand minibatches on read.
+//
+// One frame from `atlas` (the CTA's staged copy in shared memory, or the u8 atlas in global memory) and its 49 kinds.
+template <bool BLOCKED>
+__device__ __forceinline__ void render_frame(const uint8_t* atlas, const uint8_t* kp, const uint32_t (&lut)[kChunksPerLane],
+                                             uint8_t* frame, int lane) {
+  if (BLOCKED) {
+    const uint4* atlas128 = reinterpret_cast<const uint4*>(atlas);
+#pragma unroll
+    for (int k = 0; k < kChunksPerLane; ++k) {
+      const int c = lane + 32 * k;
+      if (c < kChunks) {
+        const uint32_t q = lut[k];
+        const uint4 v = atlas128[kp[q & 0xff] * (kTileBytes / 16) + (q >> 8)];
+        st_stream_v4(frame + c * 16, v.x, v.y, v.z, v.w);
+      }
+    }
+  } else {
+    blit_frame(atlas, kp, lut, frame, lane);
+  }
+}
+
 template <bool BLOCKED>
 __global__ void __launch_bounds__(256, 2) render_kernel(const RenderParams p) {
   extern __shared__ __align__(16) uint8_t smem[];
@@ -49,30 +70,24 @@ __global__ void __launch_bounds__(256, 2) render_kernel(const RenderParams p) {
       long long row = p.index ? p.index[m] : m;
       if (p.n_rows && (row < 0 || row >= p.n_rows)) row = 0;  // never read outside the buffer; callers validate indices
       const uint8_t* sym = p.sym + (size_t)row * kSymBytes;
+      bool staged = true;
 #pragma unroll
       for (int h = 0; h < 2; ++h) {
         const int k = lane + 32 * h;  // cell index vi*7 + vj, the order Grid.encode stores them
         if (k < kCells) {
           const uint32_t t = sym[3 * k], c = sym[3 * k + 1], st = sym[3 * k + 2];
-          kp[k] = (uint8_t)kind_of_sym(t, c, st, k == (kView / 2) * kView + (kView - 1));
+          const uint32_t kind = kind_of_sym(t, c, st, k == (kView / 2) * kView + (kView - 1));
+          kp[k] = (uint8_t)kind;
+          staged = staged && tile_bit(p.tile_present, kind);
         }
       }
+      // Only the tiles the current pool can show were staged.  A stored image may show others (it was stepped under an
+      // earlier pool, or never came from this handle at all): such a frame is read from the atlas in global memory.
+      const bool all_staged = __all_sync(0xffffffffu, staged);
       __syncwarp();
       uint8_t* frame = p.out + (size_t)m * kImgBytes;
-      if (BLOCKED) {
-        const uint4* atlas128 = reinterpret_cast<const uint4*>(atlas_s);
-#pragma unroll
-        for (int k = 0; k < kChunksPerLane; ++k) {
-          const int c = lane + 32 * k;
-          if (c < kChunks) {
-            const uint32_t q = lut[k];
-            const uint4 v = atlas128[kp[q & 0xff] * (kTileBytes / 16) + (q >> 8)];
-            st_stream_v4(frame + c * 16, v.x, v.y, v.z, v.w);
-          }
-        }
-      } else {
-        blit_frame(atlas_s, kp, lut, frame, lane);
-      }
+      if (all_staged) render_frame<BLOCKED>(atlas_s, kp, lut, frame, lane);
+      else render_frame<BLOCKED>(p.atlas, kp, lut, frame, lane);
       __syncwarp();  // kp is reused by this warp's next frame
     }
     __syncthreads();  // the next ticket is in shared memory
