@@ -64,7 +64,7 @@ struct merlin_env {
   // per-handle tuning knobs (-1 = follow the process-wide default) and occupancy cache
   int kernel_choice = -1;
   int observation_path = -1;
-  int occ[kOccSlots] = {};
+  OccupancyCache occ;
   // action sampler (merlin_env_policy_step)
   uint64_t sampler_seed = 0x9E3779B97F4A7C15ull;
   uint32_t* draws = nullptr;             // [N] draws made so far per env
@@ -118,7 +118,7 @@ static LaunchCtx launch_ctx(merlin_env* h) {
   c.sm_count = h->sm_count;
   c.kernel_choice = h->kernel_choice >= 0 ? h->kernel_choice : g_default_kernel_choice.load();
   c.observation_path = h->observation_path >= 0 ? h->observation_path : g_default_observation_path.load();
-  c.occ = h->occ;
+  c.occ = &h->occ;
   return c;
 }
 
@@ -628,8 +628,7 @@ int64_t merlin_env_launch_count(merlin_env_t* h) { return h ? h->launches : 0; }
 
 const char* merlin_env_step_kernel(merlin_env_t* h, int rgb) {
   if (!h) return "";
-  constexpr uint32_t kNotLean = MERLIN_F_SEVEN_ACTIONS | MERLIN_F_STUCK_PENALTY | MERLIN_F_EXPLORE_BONUS;
-  return step_kernel_name(h->cfg.n_envs, (rgb & 1) != 0, (h->cfg.flags & kNotLean) == 0, launch_ctx(h));
+  return step_kernel_name(select_step_kernel(h->cfg.n_envs, (rgb & 1) != 0, lean_config(h->cfg.flags), launch_ctx(h)));
 }
 
 static int check_kernel_choice(int choice, int lowest) {

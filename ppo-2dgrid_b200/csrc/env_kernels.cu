@@ -74,7 +74,7 @@ __global__ void __launch_bounds__(kThreads, 1) env_kernel(const EnvParams p, con
 }
 
 // ---------------------------------------------------------------------------------------------------
-// env_kernel_ordered<G, STEP, THREADS, MINB>: env_kernel's mapping (a warp owns G consecutive envs for both phases)
+// env_kernel_ordered<STEP>: env_kernel's mapping (a warp owns kOrdG consecutive envs for both phases)
 // with the groups handed out IN ORDER, one ticket per warp, from the same self-resetting counter the tile kernel
 // uses.  Every warp of the SM runs its own state phase (no warp-0 bottleneck, no CTA barrier in the loop): the
 // dependent-load chain of a state phase (~10 us) is hidden by all resident warps instead of one per CTA, while the
@@ -83,18 +83,20 @@ __global__ void __launch_bounds__(kThreads, 1) env_kernel(const EnvParams p, con
 //   G=8, 128 thr x 3 CTAs  1.046    G=16, 128 x 3  1.045    G=32, 128 x 3  1.041    G=8, 128 x 4 (spills)  1.033
 //   G=8, 256 x 2  1.034    G=16, 256 x 2  1.024    G=16, 128 x 4  1.021    G=4, 128 x 4  0.920
 // i.e. in-order hand-out lifts the group mapping from 0.92 (static assignment) to 1.05, but more concurrent state phases
-// buy nothing over the tile kernel: its limit is the store stream, not the state-phase chain.  Kept selectable (choice 6).
-template <int G, int STEP, int THREADS, int MINB, bool SWAR = false>
-__global__ void __launch_bounds__(THREADS, MINB) env_kernel_ordered(const EnvParams p, const int n_groups) {
+// buy nothing over the tile kernel: its limit is the store stream, not the state-phase chain
+// (profiles/r01_ordered_group_variants.txt).  Kept selectable (choice 6) in the first shape of the table.
+constexpr int kOrdG = 8, kOrdThreads = 128, kOrdCtas = 3;
+template <int STEP, bool SWAR = false>
+__global__ void __launch_bounds__(kOrdThreads, kOrdCtas) env_kernel_ordered(const EnvParams p, const int n_groups) {
   extern __shared__ __align__(16) uint8_t smem[];
   const int lane = threadIdx.x & 31;
   const int warp = threadIdx.x >> 5;
   Flags f(p);
   if (SWAR) f.doors = pool_has_doors(p.tile_present);
   uint8_t* atlas_s = smem;
-  uint8_t* warp_s = smem + kAtlasBytes + warp * warp_smem_bytes(G);
+  uint8_t* warp_s = smem + kAtlasBytes + warp * warp_smem_bytes(kOrdG);
   uint8_t* kinds_s = warp_s;
-  uint8_t* sym_s = warp_s + G * kKindStride;
+  uint8_t* sym_s = warp_s + kOrdG * kKindStride;
 
   uint32_t lut[kChunksPerLane];
   if (f.want_rgb) {
@@ -109,10 +111,10 @@ __global__ void __launch_bounds__(THREADS, MINB) env_kernel_ordered(const EnvPar
   while (g < n_groups) {
     int next = 0;
     if (lane == 0) next = (int)atomicAdd(&p.sched[0], 1u);
-    const int e0 = g * G;
-    const unsigned render_mask = state_phase<G, STEP, SWAR>(p, f, e0, lane, kinds_s, sym_s);
+    const int e0 = g * kOrdG;
+    const unsigned render_mask = state_phase<kOrdG, STEP, SWAR>(p, f, e0, lane, kinds_s, sym_s);
     if (f.want_sym && render_mask)
-      emit_sym_rows(p.obs_sym + (size_t)e0 * kSymBytes, sym_s, min(G, p.N - e0), render_mask, lane, 32);
+      emit_sym_rows(p.obs_sym + (size_t)e0 * kSymBytes, sym_s, min(kOrdG, p.N - e0), render_mask, lane, 32);
     if (f.want_rgb) {
       unsigned m = render_mask;
       while (m) {
@@ -125,7 +127,7 @@ __global__ void __launch_bounds__(THREADS, MINB) env_kernel_ordered(const EnvPar
     g = __shfl_sync(0xffffffffu, next, 0);
   }
   // every warp of the grid has drawn its last ticket once all of them have passed here: the last one rearms
-  if (lane == 0 && atomicAdd(&p.sched[1], 1u) == gridDim.x * (THREADS / 32) - 1) {
+  if (lane == 0 && atomicAdd(&p.sched[1], 1u) == gridDim.x * (kOrdThreads / 32) - 1) {
     p.sched[0] = 0;
     p.sched[1] = 0;
   }
@@ -140,11 +142,12 @@ __host__ __device__ constexpr int sym_kernel_warp_smem(bool swar) {
   return swar ? 32 * kSymBytes : warp_smem_bytes(32);
 }
 
-#ifndef MERLIN_SYM_MINB
-#define MERLIN_SYM_MINB 10  // 48 registers, 40 warps/SM: 1.16e10 env-steps/s at 1M envs (unconstrained, 56 registers: 1.11e10; 12 CTAs, 40 registers + spills: 1.04e10)
-#endif
+// Resident CTAs the row-parallel form is compiled for: 48 registers, 40 warps/SM, 1.16e10 env-steps/s at 1M envs
+// (unconstrained, 56 registers: 1.11e10; 12 CTAs, 40 registers + spills: 1.04e10;
+// profiles/r01_symbolic_kernel_occupancy_variants.txt).
+constexpr int kSymSwarCtas = 10;
 template <int STEP, bool SWAR = false>
-__global__ void __launch_bounds__(128, SWAR ? MERLIN_SYM_MINB : 1) env_kernel_sym(const EnvParams p, const int n_groups) {
+__global__ void __launch_bounds__(128, SWAR ? kSymSwarCtas : 1) env_kernel_sym(const EnvParams p, const int n_groups) {
   extern __shared__ __align__(16) uint8_t smem[];
   const int lane = threadIdx.x & 31;
   const int warp = threadIdx.x >> 5;
@@ -176,111 +179,103 @@ static cudaError_t launch_sym_kernel(const EnvParams& p, const LaunchCtx& ctx, c
 }
 
 // ---------------------------------------------------------------------------------------------------
-// launch helpers: persistent grids of (SMs x resident CTAs), capped by the work available (resident_ctas and the
-// occupancy-cache slots: env_kernels_common.cuh).
+// launch helpers: persistent grids of (SMs x resident CTAs), capped by the work available (resident_ctas:
+// env_kernels_common.cuh).
 template <int G, int STEP>
 static cudaError_t launch_group_kernel(const EnvParams& p, const LaunchCtx& ctx, cudaStream_t stream) {
   const int n_groups = (p.N + G - 1) / G;
   const size_t smem = cta_smem_bytes(G);
-  int& blocks_per_sm = ctx.occ[kSlotGroup + 3 * (G == 32 ? 0 : G == 16 ? 1 : G == 8 ? 2 : 3) + STEP];
-  if (!blocks_per_sm) {
-    cudaError_t err = resident_ctas(env_kernel<G, STEP>, kThreads, smem, blocks_per_sm);
-    if (err != cudaSuccess) return err;
-  }
-  const int grid = min(ctx.sm_count * blocks_per_sm, (n_groups + kWarps - 1) / kWarps);
+  int ctas;
+  if (cudaError_t err = resident_ctas(ctx, env_kernel<G, STEP>, kThreads, smem, ctas)) return err;
+  const int grid = min(ctx.sm_count * ctas, (n_groups + kWarps - 1) / kWarps);
   env_kernel<G, STEP><<<grid, kThreads, smem, stream>>>(p, n_groups);
   return cudaGetLastError();
 }
 
-#ifndef MERLIN_ORD_G
-#define MERLIN_ORD_G 8
-#define MERLIN_ORD_THREADS 128
-#define MERLIN_ORD_CTAS 3
-#endif
-template <int G, int STEP, bool SWAR, int THREADS = MERLIN_ORD_THREADS, int MINB = MERLIN_ORD_CTAS>
+template <int STEP, bool SWAR>
 static cudaError_t launch_ordered_kernel_impl(const EnvParams& p, const LaunchCtx& ctx, cudaStream_t stream) {
-  constexpr int warps = THREADS / 32;
-  const int n_groups = (p.N + G - 1) / G;
-  const size_t smem = kAtlasBytes + warps * warp_smem_bytes(G);
-  int& blocks_per_sm = ctx.occ[kSlotOrdered + (SWAR ? 3 : 0) + STEP];
-  if (!blocks_per_sm) {
-    cudaError_t err = resident_ctas(env_kernel_ordered<G, STEP, THREADS, MINB, SWAR>, THREADS, smem, blocks_per_sm);
-    if (err != cudaSuccess) return err;
-    if (MINB < blocks_per_sm) blocks_per_sm = MINB;
-  }
-  const int grid = min(ctx.sm_count * blocks_per_sm, (n_groups + warps - 1) / warps);
-  env_kernel_ordered<G, STEP, THREADS, MINB, SWAR><<<grid, THREADS, smem, stream>>>(p, n_groups);
+  constexpr int warps = kOrdThreads / 32;
+  const int n_groups = (p.N + kOrdG - 1) / kOrdG;
+  const size_t smem = kAtlasBytes + warps * warp_smem_bytes(kOrdG);
+  int ctas;
+  if (cudaError_t err = resident_ctas(ctx, env_kernel_ordered<STEP, SWAR>, kOrdThreads, smem, ctas, kOrdCtas))
+    return err;
+  const int grid = min(ctx.sm_count * ctas, (n_groups + warps - 1) / warps);
+  env_kernel_ordered<STEP, SWAR><<<grid, kOrdThreads, smem, stream>>>(p, n_groups);
   return cudaGetLastError();
 }
-template <int G, int STEP>
+template <int STEP>
 static cudaError_t launch_ordered_kernel(const EnvParams& p, const LaunchCtx& ctx, cudaStream_t stream) {
-  return use_swar(p, ctx, true) ? launch_ordered_kernel_impl<G, STEP, true>(p, ctx, stream)
-                                : launch_ordered_kernel_impl<G, STEP, false>(p, ctx, stream);
+  return use_swar(p, ctx, true) ? launch_ordered_kernel_impl<STEP, true>(p, ctx, stream)
+                                : launch_ordered_kernel_impl<STEP, false>(p, ctx, stream);
 }
 
-#ifndef MERLIN_TILE16_MIN_ENVS
-#define MERLIN_TILE16_MIN_ENVS(SMS) ((SMS) * kTileCtasPerSm * 16)
-#endif
-constexpr int kSymWarpMaxEnvs = 2048;   // symbolic-only batches up to this size run the warp-per-env kernel
+// Automatic choice, from the B200 sweeps in profiles/.  RGB observations: the warp kernel while every env of the batch
+// is resident at once or nearly so, the tile kernel above.  The quad kernel (choice 7) is not picked: under CUDA-graph
+// replay it is 7 % faster at 8192 envs (14.6 vs 15.7 us), equal at 5120-6144, slower below (8.8 vs 8.3 us at 4096) and
+// above (22.4 vs 20.6 us at 12 288), and slower everywhere when launched eagerly (profiles/r02_quad_vs_warp.txt).
+// Symbolic-only observations are instruction-bound: the state phase alone, at high occupancy -- except for batches so
+// small that one env's chain of ~1800 dependent instructions IS the run time: there a warp per env (the same chain
+// spread over 32 lanes) is 1.3 us faster (2.9 vs 4.2 us at 32 envs, 3.4 vs 4.7 us at 1024; equal at ~3000).
+constexpr int kRgbWarpMaxEnvs = 24576;
+constexpr int kSymWarpMaxEnvs = 2048;
+
+StepKernel select_step_kernel(int n_envs, bool rgb, bool lean, const LaunchCtx& ctx) {
+  int choice = ctx.kernel_choice;
+  if (choice == kChoiceAuto) {
+    if (rgb) choice = n_envs <= kRgbWarpMaxEnvs ? kChoiceWarp : kChoiceTile;
+    else choice = n_envs <= kSymWarpMaxEnvs ? kChoiceWarp : kChoiceSym;
+  }
+  switch (choice) {
+    case kChoiceGroup: {
+      // the largest group size that still yields >= ~8 warps per SM; tiny batches use smaller groups
+      const long long want_warps = (long long)ctx.sm_count * 8;
+      for (int G = 32; G > 4; G /= 2)
+        if (n_envs / G >= want_warps) return {kChoiceGroup, G};
+      return {kChoiceGroup, 4};
+    }
+    case kChoiceTile:
+      // tiles of 16 envs once every resident CTA gets one; smaller tiles spread a small batch over more CTAs
+      return {kChoiceTile, n_envs >= ctx.sm_count * kTileCtasPerSm * 16 ? 16 : 8};
+    case kChoiceQuad:
+      return {lean && rgb ? kChoiceQuad : kChoiceWarp, 0};
+    default:
+      return {choice, 0};
+  }
+}
+
+const char* step_kernel_name(StepKernel k) {
+  switch (k.choice) {
+    case kChoiceGroup:
+      return k.size == 32 ? "merlin::env_kernel<32,true>" : k.size == 16 ? "merlin::env_kernel<16,true>"
+           : k.size == 8  ? "merlin::env_kernel<8,true>"  : "merlin::env_kernel<4,true>";
+    case kChoiceTile: return k.size == 16 ? "merlin::env_kernel_tile<16,true>" : "merlin::env_kernel_tile<8,true>";
+    case kChoiceTileTma: return "merlin::env_kernel_tile_tma<true>";
+    case kChoiceSym: return "merlin::env_kernel_sym<true>";
+    case kChoiceOrdered: return "merlin::env_kernel_ordered<true>";
+    case kChoiceQuad: return "merlin::env_kernel_quad<true>";
+    default: return "merlin::env_kernel_warp<true>";
+  }
+}
 
 template <int STEP>
 static cudaError_t launch_sized(const EnvParams& p, const LaunchCtx& ctx, cudaStream_t stream) {
-  const int sm_count = ctx.sm_count;
-  int choice = ctx.kernel_choice;
-  if (choice == 0) {
-    // symbolic-only observations are instruction-bound: the state phase alone, at high occupancy -- except for batches so
-    // small that one env's chain of ~1800 dependent instructions IS the run time: there a warp per env (the same chain
-    // spread over 32 lanes) is 1.3 us faster (2.9 vs 4.2 us at 32 envs, 3.4 vs 4.7 us at 1024; equal at ~3000)
-    if (p.obs_rgb == nullptr) choice = p.N <= kSymWarpMaxEnvs ? 2 : 5;
-    else choice = MERLIN_AUTO_RGB_CHOICE(p.N, sm_count);
+  const StepKernel k = select_step_kernel(p.N, p.obs_rgb != nullptr, lean_config(p.flags), ctx);
+  switch (k.choice) {
+    case kChoiceGroup:
+      if (k.size == 32) return launch_group_kernel<32, STEP>(p, ctx, stream);
+      if (k.size == 16) return launch_group_kernel<16, STEP>(p, ctx, stream);
+      if (k.size == 8) return launch_group_kernel<8, STEP>(p, ctx, stream);
+      return launch_group_kernel<4, STEP>(p, ctx, stream);
+    case kChoiceTile: return launch_tile_kernel(k.size, STEP, p, ctx, stream);
+    case kChoiceTileTma: return launch_tile_tma_kernel(STEP, p, ctx, stream);
+    case kChoiceSym: return launch_sym_kernel<STEP>(p, ctx, stream);
+    case kChoiceOrdered: return launch_ordered_kernel<STEP>(p, ctx, stream);
+    case kChoiceQuad:
+      if (STEP != 0) return launch_quad_kernel(STEP, p, ctx, stream);
+      return launch_warp_kernel(STEP, p, ctx, stream);   // the quad kernel only steps
+    default: return launch_warp_kernel(STEP, p, ctx, stream);
   }
-  if (choice == 2 && ctx.kernel_choice == 0 && MERLIN_AUTO_QUAD(p.N)) choice = 7;   // quads where they apply and win
-  if (choice == 7) {
-    if (STEP != 0 && quad_eligible(p)) return launch_quad_kernel(STEP, p, ctx, stream);
-    choice = 2;
-  }
-  if (choice == 2) return launch_warp_kernel(STEP, p, ctx, stream);
-  if (choice == 5) return launch_sym_kernel<STEP>(p, ctx, stream);
-  if (choice == 6) return launch_ordered_kernel<MERLIN_ORD_G, STEP>(p, ctx, stream);
-  if (choice == 4) {
-    if ((reinterpret_cast<uintptr_t>(p.obs_rgb) & 15) == 0) return launch_tile_tma_kernel(STEP, p, ctx, stream);
-    choice = 3;  // bulk copies need a 16-byte aligned destination
-  }
-  if (choice == 3) {
-    // tiles of 16 envs once every resident CTA gets one; smaller tiles spread a small batch over more CTAs
-    if (p.N >= MERLIN_TILE16_MIN_ENVS(sm_count)) return launch_tile_kernel(16, STEP, p, ctx, stream);
-    return launch_tile_kernel(8, STEP, p, ctx, stream);
-  }
-  // pick the largest group size that still yields >= ~8 warps per SM; tiny batches use smaller groups
-  const long long want_warps = (long long)sm_count * 8;
-  if (p.N / 32 >= want_warps) return launch_group_kernel<32, STEP>(p, ctx, stream);
-  if (p.N / 16 >= want_warps) return launch_group_kernel<16, STEP>(p, ctx, stream);
-  if (p.N / 8 >= want_warps) return launch_group_kernel<8, STEP>(p, ctx, stream);
-  return launch_group_kernel<4, STEP>(p, ctx, stream);
-}
-
-const char* step_kernel_name(int n_envs, bool rgb, bool quad_ok, const LaunchCtx& ctx) {
-  const int sm_count = ctx.sm_count;
-  int choice = ctx.kernel_choice;
-  if (choice == 0) {
-    choice = rgb ? MERLIN_AUTO_RGB_CHOICE(n_envs, sm_count) : (n_envs <= kSymWarpMaxEnvs ? 2 : 5);
-    if (choice == 2 && rgb && MERLIN_AUTO_QUAD(n_envs)) choice = 7;
-  }
-  if (choice == 7) {
-    if (quad_ok && rgb) return "merlin::env_kernel_quad<true>";
-    choice = 2;
-  }
-  if (choice == 5) return "merlin::env_kernel_sym<true>";
-  if (choice == 2) return "merlin::env_kernel_warp<true>";
-  if (choice == 4) return "merlin::env_kernel_tile_tma<true>";
-  if (choice == 6) return "merlin::env_kernel_ordered<true>";
-  if (choice == 3)
-    return n_envs >= MERLIN_TILE16_MIN_ENVS(sm_count) ? "merlin::env_kernel_tile<16,true>" : "merlin::env_kernel_tile<8,true>";
-  const long long want_warps = (long long)sm_count * 8;
-  if (n_envs / 32 >= want_warps) return "merlin::env_kernel<32,true>";
-  if (n_envs / 16 >= want_warps) return "merlin::env_kernel<16,true>";
-  if (n_envs / 8 >= want_warps) return "merlin::env_kernel<8,true>";
-  return "merlin::env_kernel<4,true>";
 }
 
 cudaError_t launch_env_step(const EnvParams& p, const LaunchCtx& ctx, cudaStream_t stream) {

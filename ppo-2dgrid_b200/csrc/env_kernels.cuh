@@ -9,16 +9,6 @@
 namespace merlin {
 
 constexpr int kThreads = 256;                 // 8 warps per CTA
-// automatic kernel choice for RGB observations (1 group / 2 warp / 3 tile), from the B200 sweep in profiles/
-#ifndef MERLIN_AUTO_RGB_CHOICE
-#define MERLIN_AUTO_RGB_CHOICE(N, SMS) ((N) <= 24576 ? 2 : 3)
-#endif
-// Would the automatic choice 2 become 7 (env_kernel_quad) at N envs?  Measured and NOT adopted: under CUDA-graph replay
-// it is 7 % faster at 8192 envs (14.6 vs 15.7 us), equal at 5120-6144, slower below (8.8 vs 8.3 us at 4096) and above
-// (22.4 vs 20.6 us at 12 288), and slower everywhere when launched eagerly (profiles/r02_quad_vs_warp.txt).
-#ifndef MERLIN_AUTO_QUAD
-#define MERLIN_AUTO_QUAD(N) 0
-#endif
 constexpr int kWarps = kThreads / 32;
 constexpr int kAtlasBytes = kAtlasTiles * kTileBytes;   // 24576
 constexpr int kKindStride = 52;               // 49 tile kinds per env, padded: odd word stride -> conflict-free lanes
@@ -78,24 +68,54 @@ struct EnvParams {
   uint8_t* rec_goal;           // [N] 1 = the episode ended by termination with a positive reward (goal reached)
 };
 
-// Per-handle launch context: kernel choice, observation path and the occupancy cache live in the handle (a process may
-// hold several handles on several devices, driven from different threads).
-constexpr int kOccSlots = 44;
-struct LaunchCtx {
-  int sm_count;
-  int kernel_choice;      // 0 = automatic, 1..6 as merlin_set_kernel_choice
-  int observation_path;   // 0 = automatic, 1 = per-cell, 2 = row-parallel wherever built
-  int* occ;               // [kOccSlots] resident CTAs per SM per kernel instance, 0 = not configured yet
+// Resident CTAs per SM of every kernel instance a handle has launched eagerly, keyed by the kernel's address (graph
+// replays run no host code).  Filled on first use by resident_ctas (env_kernels_common.cuh); the step kernels have
+// fewer than 50 instances.
+struct OccupancyCache {
+  static constexpr int kEntries = 64;
+  const void* kernel[kEntries] = {};
+  int ctas[kEntries] = {};
+  int n = 0;
 };
 
-// kernel choice: 0 = automatic, 1 = env_kernel (warp owns a group), 2 = env_kernel_warp (warp per env), 3 = env_kernel_tile,
-// 4 = env_kernel_tile_tma (tile kernel, frames through cp.async.bulk), 5 = env_kernel_sym (state phase only: any RGB
-// output pointer is ignored), 6 = env_kernel_ordered (group kernel, groups handed out in order), 7 = env_kernel_quad (four
-// envs per warp; steps of the lean configuration with RGB frames -- anything else asked of it runs choice 2)
+// Per-handle launch context: kernel choice, observation path and the occupancy cache live in the handle (a process may
+// hold several handles on several devices, driven from different threads).
+struct LaunchCtx {
+  int sm_count;
+  int kernel_choice;      // 0 = automatic, 1..7 as merlin_set_kernel_choice
+  int observation_path;   // 0 = automatic, 1 = per-cell, 2 = row-parallel wherever built
+  OccupancyCache* occ;
+};
+
+// kernel choice (merlin_set_kernel_choice)
+enum KernelChoice : int {
+  kChoiceAuto = 0,
+  kChoiceGroup = 1,     // env_kernel<G>: a warp owns a group of G envs
+  kChoiceWarp = 2,      // env_kernel_warp: a warp per env
+  kChoiceTile = 3,      // env_kernel_tile<T>: a CTA owns a tile of T envs
+  kChoiceTileTma = 4,   // env_kernel_tile_tma: the tile kernel with its frames stored through cp.async.bulk
+  kChoiceSym = 5,       // env_kernel_sym: state phase only -- any RGB output pointer is ignored
+  kChoiceOrdered = 6,   // env_kernel_ordered: the group kernel with groups handed out in order
+  kChoiceQuad = 7,      // env_kernel_quad: four envs per warp; steps of the lean configuration with RGB frames --
+                        // anything else asked of it runs kChoiceWarp
+};
 // observation path: 0 = automatic (row-parallel obs_swar.cuh in the symbolic-only kernel when W >= 7), 1 = per-cell
 // everywhere, 2 = row-parallel in every kernel that has it (symbolic-only, tile, ordered)
-// quad_ok: three actions, no shaping wrapper (what env_kernel_quad serves)
-const char* step_kernel_name(int n_envs, bool rgb, bool quad_ok, const LaunchCtx& ctx);
+
+// The lean configuration (the reference's own): three actions (=> immutable grids), no stuck penalty, no exploration
+// bonus.  The quad kernel and the lean form of the warp kernel serve only this configuration.
+inline bool lean_config(uint32_t flags) {
+  return (flags & (MERLIN_F_SEVEN_ACTIONS | MERLIN_F_STUCK_PENALTY | MERLIN_F_EXPLORE_BONUS)) == 0;
+}
+
+// The step kernel a step of n_envs envs runs: `choice` is never kChoiceAuto, `size` is G (kChoiceGroup) or T
+// (kChoiceTile) and 0 otherwise.  A reset sent to kChoiceQuad runs kChoiceWarp.
+struct StepKernel {
+  int choice;
+  int size;
+};
+StepKernel select_step_kernel(int n_envs, bool rgb, bool lean, const LaunchCtx& ctx);
+const char* step_kernel_name(StepKernel k);
 cudaError_t launch_env_step(const EnvParams& p, const LaunchCtx& ctx, cudaStream_t stream);
 cudaError_t launch_env_reset(const EnvParams& p, const LaunchCtx& ctx, cudaStream_t stream);
 // Frames from stored symbolic observations (RGBImgPartialObsWrapper.observation as a batch op, with an optional

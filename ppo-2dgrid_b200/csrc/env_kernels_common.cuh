@@ -170,27 +170,37 @@ __device__ __forceinline__ void emit_sym_rows(uint8_t* out, const uint8_t* sym_s
 }
 
 // ---------------------------------------------------------------------------------------------------
-// launch helpers: persistent grids of (SMs x resident CTAs), capped by the work available.  The resident-CTA count of
-// every kernel instance is looked up once per HANDLE (LaunchCtx::occ, one slot per instance): a process may drive
-// several handles on several devices from several threads, so nothing here is process-wide.
+// launch helper: resident CTAs per SM of `kernel` launched with `threads` threads and `smem` bytes of dynamic shared
+// memory, at most `max_ctas` -- the persistent kernels launch SMs x that many CTAs, capped by the work available.  The
+// first launch of an instance through a handle sets its shared-memory attribute and queries the occupancy; the count is
+// kept in the HANDLE's cache (LaunchCtx::occ): a process may drive several handles on several devices from several
+// threads, so nothing here is process-wide.
 template <typename Kernel>
-static cudaError_t resident_ctas(Kernel kernel, int threads, size_t smem, int& blocks_per_sm) {
+static cudaError_t resident_ctas(const LaunchCtx& ctx, Kernel kernel, int threads, size_t smem, int& ctas,
+                                 int max_ctas = 1 << 30) {
+  OccupancyCache& c = *ctx.occ;
+  const void* key = reinterpret_cast<const void*>(kernel);
+  for (int i = 0; i < c.n; ++i) {
+    if (c.kernel[i] == key) {
+      ctas = c.ctas[i];
+      return cudaSuccess;
+    }
+  }
   cudaError_t err = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
   if (err != cudaSuccess) return err;
-  err = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&blocks_per_sm, kernel, threads, smem);
+  err = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&ctas, kernel, threads, smem);
   if (err != cudaSuccess) return err;
-  if (blocks_per_sm < 1) blocks_per_sm = 1;
+  ctas = max(1, min(ctas, max_ctas));
+  if (c.n < OccupancyCache::kEntries) {
+    c.kernel[c.n] = key;
+    c.ctas[c.n] = ctas;
+    c.n += 1;
+  }
   return cudaSuccess;
 }
-
-// occupancy-cache slots (LaunchCtx::occ): one per kernel instance
-enum : int { kSlotGroup = 0 /* + 3*log2(32/G) + STEP: 12 */, kSlotTile = 12 /* + (T==8)*6 + SWAR*3 + STEP: 12 */,
-             kSlotOrdered = 24 /* + SWAR*3 + STEP: 6 */, kSlotTma = 30 /* + STEP: 3 */, kSlotWarp = 33 /* + LEAN*3 + STEP: 6 */, kSlotQuad = 39 /* + STEP - 1: 2 */ };
-static_assert(kSlotQuad + 2 <= kOccSlots, "occupancy cache too small");
 
 // small-batch step kernels (env_kernels_small.cu); `step` = 0 masked reset, 1 step with given actions, 2 policy step
 cudaError_t launch_warp_kernel(int step, const EnvParams& p, const LaunchCtx& ctx, cudaStream_t stream);
 cudaError_t launch_quad_kernel(int step, const EnvParams& p, const LaunchCtx& ctx, cudaStream_t stream);   // step 1 or 2
-bool quad_eligible(const EnvParams& p);
 
 }  // namespace merlin

@@ -29,20 +29,14 @@ namespace merlin {
 //     588-entry chunk map (ncu at 4096 envs, profiles/r02_warp_n4096_v2_ncu_details.csv: 1387 -> 791 warp instructions per env).
 //     The kinds are kept premultiplied (kind * 192, the tile's byte offset in the atlas) as 16-bit words.
 //   * atlas staging touches only the slots the pool can show: thread t tests tile t / 2 and copies half of it.
-#ifndef MERLIN_WARP_THREADS
-#define MERLIN_WARP_THREADS 256
-#define MERLIN_WARP_CTAS 4
-#endif
+constexpr int kWarpKernelThreads = 256, kWarpCtas = 4;
 // RGB batches of at least this many envs launch the warp kernel with programmatic dependent launch (see the kernel)
-#ifndef MERLIN_WARP_PDL_MIN_ENVS
-#define MERLIN_WARP_PDL_MIN_ENVS 4096
-#endif
-constexpr int kWarpKernelThreads = MERLIN_WARP_THREADS;
+constexpr int kWarpPdlMinEnvs = 4096;
 constexpr int kWarpKindBytes = 128;          // 49 premultiplied kinds (u16) per warp, padded
 constexpr int kPairChunks = 2 * kUnitsPerRow / 2;   // 21 16-byte chunks per pair of pixel rows
 
 template <int STEP, bool PDL, bool LEAN = false>
-__global__ void __launch_bounds__(kWarpKernelThreads, MERLIN_WARP_CTAS) env_kernel_warp(const EnvParams p) {
+__global__ void __launch_bounds__(kWarpKernelThreads, kWarpCtas) env_kernel_warp(const EnvParams p) {
   extern __shared__ __align__(16) uint8_t smem[];
   const int lane = threadIdx.x & 31;
   const int warp = threadIdx.x >> 5;
@@ -329,9 +323,7 @@ __global__ void __launch_bounds__(kWarpKernelThreads, MERLIN_WARP_CTAS) env_kern
 //   * frame phase as in env_kernel_warp (map-free row pairs), one env after the other.
 // Quads are dealt to warps CTA-minor (quad q -> warp q / gridDim of CTA q % gridDim), so a batch that needs 1.3 rounds
 // leaves every SM with the same share of second-round quads.
-#ifndef MERLIN_QUAD_CTAS
-#define MERLIN_QUAD_CTAS 4
-#endif
+constexpr int kQuadCtas = 4;
 constexpr int kQuadKindBytes = 4 * 128 + 32;   // per warp: 4 envs x 49 premultiplied kinds (u16, padded to 64) + 4 x 8 row masks
 
 // Row `r` (0 = farthest, 7 = the agent's own row) of the 8 x 7 region in front of pose (x, y, heading f): codes of its
@@ -355,7 +347,7 @@ __device__ __forceinline__ void load_ext_row(const EnvParams& p, const uint8_t* 
 }
 
 template <int STEP, bool PDL>
-__global__ void __launch_bounds__(kWarpKernelThreads, MERLIN_QUAD_CTAS) env_kernel_quad(const EnvParams p) {
+__global__ void __launch_bounds__(kWarpKernelThreads, kQuadCtas) env_kernel_quad(const EnvParams p) {
   static_assert(STEP == 1 || STEP == 2, "the quad kernel steps; resets run the warp kernel");
   extern __shared__ __align__(16) uint8_t smem[];
   const int lane = threadIdx.x & 31;
@@ -533,14 +525,11 @@ __global__ void __launch_bounds__(kWarpKernelThreads, MERLIN_QUAD_CTAS) env_kern
 // and the launch lasts as long as the SMs with 32.  Instead the CTA shape follows the batch: the fewest envs per SM
 // that cover it, ceil(N / SMs), split into c <= resident CTAs of w <= 8 warps (4096 envs: 4 x 7 warps, 28 envs on
 // (almost) every SM).  Larger batches loop over rounds of full CTAs, where the imbalance is a few percent at most.
-#ifndef MERLIN_WARP_BALANCE
-#define MERLIN_WARP_BALANCE 1
-#endif
 static void warp_kernel_shape(int N, int sm_count, int blocks_per_sm, int& grid, int& threads, bool few_ctas = false) {
   constexpr int max_warps = kWarpKernelThreads / 32;
   threads = kWarpKernelThreads;
   grid = min(sm_count * blocks_per_sm, (N + max_warps - 1) / max_warps);
-  if (!MERLIN_WARP_BALANCE || N > sm_count * blocks_per_sm * max_warps) return;
+  if (N > sm_count * blocks_per_sm * max_warps) return;
   const int per_sm = (N + sm_count - 1) / sm_count;
   int best_w = max_warps, best_cost = 1 << 30;
   for (int c = blocks_per_sm; c >= 1; --c) {   // ties: more, smaller CTAs (each clears its staging barrier sooner)
@@ -552,62 +541,6 @@ static void warp_kernel_shape(int N, int sm_count, int blocks_per_sm, int& grid,
   grid = (N + best_w - 1) / best_w;
 }
 
-template <int STEP, bool LEAN>
-static cudaError_t launch_warp_kernel_impl(const EnvParams& p, const LaunchCtx& ctx, cudaStream_t stream) {
-  constexpr int warps = kWarpKernelThreads / 32;
-  const size_t smem = kAtlasBytes + warps * kWarpKindBytes;
-  int& blocks_per_sm = ctx.occ[kSlotWarp + (LEAN ? 3 : 0) + STEP];
-  if (!blocks_per_sm) {
-    cudaError_t err = resident_ctas(env_kernel_warp<STEP, false, LEAN>, kWarpKernelThreads, smem, blocks_per_sm);
-    if (err == cudaSuccess) {
-      int same = 0;
-      err = resident_ctas(env_kernel_warp<STEP, true, LEAN>, kWarpKernelThreads, smem, same);
-    }
-    if (err != cudaSuccess) { blocks_per_sm = 0; return err; }
-  }
-  int grid, threads;
-  warp_kernel_shape(p.N, ctx.sm_count, blocks_per_sm, grid, threads);
-  if (p.obs_rgb != nullptr && p.N >= MERLIN_WARP_PDL_MIN_ENVS) {
-    cudaLaunchConfig_t cfg = {};
-    cfg.gridDim = dim3(grid); cfg.blockDim = dim3(threads); cfg.dynamicSmemBytes = smem; cfg.stream = stream;
-    cudaLaunchAttribute attr[1];
-    attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    attr[0].val.programmaticStreamSerializationAllowed = 1;
-    cfg.attrs = attr; cfg.numAttrs = 1;
-    return cudaLaunchKernelEx(&cfg, env_kernel_warp<STEP, true, LEAN>, p);
-  }
-  env_kernel_warp<STEP, false, LEAN><<<grid, threads, smem, stream>>>(p);
-  return cudaGetLastError();
-}
-// The lean step (two dependent round trips, see the kernel) serves the reference's own configuration: three actions
-// (=> immutable grids) and no reward-shaping wrapper.
-#ifndef MERLIN_WARP_LEAN
-#define MERLIN_WARP_LEAN 1
-#endif
-// ... while every env of the batch is resident at once or nearly so: from 16 384 envs up (3.5 rounds of resident warps,
-// chains hidden behind other warps' stores) the lean form's 56-cell region and shuffles cost 1.5 % (27.5 vs 27.0 us)
-#ifndef MERLIN_WARP_LEAN_MAX_ENVS
-#define MERLIN_WARP_LEAN_MAX_ENVS 12288
-#endif
-template <int STEP>
-static cudaError_t launch_warp_kernel_step(const EnvParams& p, const LaunchCtx& ctx, cudaStream_t stream) {
-  constexpr uint32_t kNotLean = MERLIN_F_SEVEN_ACTIONS | MERLIN_F_STUCK_PENALTY | MERLIN_F_EXPLORE_BONUS;
-  if (MERLIN_WARP_LEAN && p.N <= MERLIN_WARP_LEAN_MAX_ENVS && STEP != 0 && (p.flags & kNotLean) == 0 && p.cells == nullptr)
-    return launch_warp_kernel_impl<STEP, STEP != 0>(p, ctx, stream);
-  return launch_warp_kernel_impl<STEP, false>(p, ctx, stream);
-}
-
-// env_kernel_quad serves steps of the lean configuration with RGB frames; anything else asked of choice 7 runs the warp kernel.
-bool quad_eligible(const EnvParams& p) {
-  constexpr uint32_t kNotLean = MERLIN_F_SEVEN_ACTIONS | MERLIN_F_STUCK_PENALTY | MERLIN_F_EXPLORE_BONUS;
-  return (p.flags & kNotLean) == 0 && p.cells == nullptr && p.obs_rgb != nullptr;
-}
-// The quad kernel is launched with programmatic dependent launch only when its CTAs fill every resident slot of the
-// machine: a grid that leaves room lets its successors (which signal launch_dependents on entry themselves) pile up
-// resident behind it, and a step then takes twice as long (4096 envs = 147 CTAs: 16 us instead of 9).
-#ifndef MERLIN_QUAD_PDL_MIN_ENVS
-#define MERLIN_QUAD_PDL_MIN_ENVS 16384
-#endif
 template <typename Kernel>
 static cudaError_t launch_maybe_pdl(Kernel kernel, bool pdl, int grid, int threads, size_t smem, cudaStream_t stream,
                                     const EnvParams& p) {
@@ -619,25 +552,44 @@ static cudaError_t launch_maybe_pdl(Kernel kernel, bool pdl, int grid, int threa
   cfg.attrs = attr; cfg.numAttrs = pdl ? 1 : 0;
   return cudaLaunchKernelEx(&cfg, kernel, p);
 }
+
+template <int STEP, bool LEAN>
+static cudaError_t launch_warp_kernel_impl(const EnvParams& p, const LaunchCtx& ctx, cudaStream_t stream) {
+  const size_t smem = kAtlasBytes + (kWarpKernelThreads / 32) * kWarpKindBytes;
+  const bool pdl = p.obs_rgb != nullptr && p.N >= kWarpPdlMinEnvs;
+  const auto kernel = pdl ? env_kernel_warp<STEP, true, LEAN> : env_kernel_warp<STEP, false, LEAN>;
+  int ctas;
+  if (cudaError_t err = resident_ctas(ctx, kernel, kWarpKernelThreads, smem, ctas)) return err;
+  int grid, threads;
+  warp_kernel_shape(p.N, ctx.sm_count, ctas, grid, threads);
+  return launch_maybe_pdl(kernel, pdl, grid, threads, smem, stream, p);
+}
+// The lean step (two dependent round trips, see the kernel) serves the lean configuration (lean_config) while every env
+// of the batch is resident at once or nearly so: from 16 384 envs up (3.5 rounds of resident warps, chains hidden behind
+// other warps' stores) the lean form's 56-cell region and shuffles cost 1.5 % (27.5 vs 27.0 us).
+constexpr int kWarpLeanMaxEnvs = 12288;
+template <int STEP>
+static cudaError_t launch_warp_kernel_step(const EnvParams& p, const LaunchCtx& ctx, cudaStream_t stream) {
+  if constexpr (STEP != 0) {
+    if (p.N <= kWarpLeanMaxEnvs && lean_config(p.flags)) return launch_warp_kernel_impl<STEP, true>(p, ctx, stream);
+  }
+  return launch_warp_kernel_impl<STEP, false>(p, ctx, stream);
+}
+
+// The quad kernel is launched with programmatic dependent launch only when its CTAs fill every resident slot of the
+// machine: a grid that leaves room lets its successors (which signal launch_dependents on entry themselves) pile up
+// resident behind it, and a step then takes twice as long (4096 envs = 147 CTAs: 16 us instead of 9).
+constexpr int kQuadPdlMinEnvs = 16384;
 template <int STEP>
 static cudaError_t launch_quad_kernel_step(const EnvParams& p, const LaunchCtx& ctx, cudaStream_t stream) {
-  constexpr int warps = kWarpKernelThreads / 32;
-  const size_t smem = kAtlasBytes + warps * kQuadKindBytes;
-  int& blocks_per_sm = ctx.occ[kSlotQuad + STEP - 1];
-  if (!blocks_per_sm) {
-    cudaError_t err = resident_ctas(env_kernel_quad<STEP, false>, kWarpKernelThreads, smem, blocks_per_sm);
-    if (err == cudaSuccess) {
-      int same = 0;
-      err = resident_ctas(env_kernel_quad<STEP, true>, kWarpKernelThreads, smem, same);
-    }
-    if (err != cudaSuccess) { blocks_per_sm = 0; return err; }
-    if (MERLIN_QUAD_CTAS < blocks_per_sm) blocks_per_sm = MERLIN_QUAD_CTAS;
-  }
+  const size_t smem = kAtlasBytes + (kWarpKernelThreads / 32) * kQuadKindBytes;
+  const bool pdl = p.N >= kQuadPdlMinEnvs;
+  const auto kernel = pdl ? env_kernel_quad<STEP, true> : env_kernel_quad<STEP, false>;
+  int ctas;
+  if (cudaError_t err = resident_ctas(ctx, kernel, kWarpKernelThreads, smem, ctas, kQuadCtas)) return err;
   int grid, threads;
-  warp_kernel_shape((p.N + 3) >> 2, ctx.sm_count, blocks_per_sm, grid, threads, /*few_ctas=*/true);   // one warp per quad
-  if (p.N >= MERLIN_QUAD_PDL_MIN_ENVS)
-    return launch_maybe_pdl(env_kernel_quad<STEP, true>, true, grid, threads, smem, stream, p);
-  return launch_maybe_pdl(env_kernel_quad<STEP, false>, false, grid, threads, smem, stream, p);
+  warp_kernel_shape((p.N + 3) >> 2, ctx.sm_count, ctas, grid, threads, /*few_ctas=*/true);   // one warp per quad
+  return launch_maybe_pdl(kernel, pdl, grid, threads, smem, stream, p);
 }
 
 cudaError_t launch_warp_kernel(int step, const EnvParams& p, const LaunchCtx& ctx, cudaStream_t stream) {

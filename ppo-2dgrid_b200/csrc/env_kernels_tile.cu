@@ -28,8 +28,8 @@ __host__ __device__ constexpr int tile_smem_bytes(int T) {
   return kAtlasBytes + ((T * kKindStride + T * kSymBytes + 15) & ~15) + 16;
 }
 
-template <int T, int STEP, int THREADS = kTileThreads, int MINB = kTileCtasPerSm, bool SWAR = false>
-__global__ void __launch_bounds__(THREADS, MINB) env_kernel_tile(const EnvParams p, const int n_tiles) {
+template <int T, int STEP, bool SWAR = false>
+__global__ void __launch_bounds__(kTileThreads, kTileCtasPerSm) env_kernel_tile(const EnvParams p, const int n_tiles) {
   extern __shared__ __align__(16) uint8_t smem[];
   const int lane = threadIdx.x & 31;
   const int warp = threadIdx.x >> 5;
@@ -84,8 +84,8 @@ __global__ void __launch_bounds__(THREADS, MINB) env_kernel_tile(const EnvParams
 }
 
 // ---------------------------------------------------------------------------------------------------
-// env_kernel_tile_tma<T, STEP, THREADS, MINB, NBUF>: env_kernel_tile with the frame phase routed through the TMA unit.
-// A warp assembles a frame in one of its NBUF shared-memory staging buffers (the same atlas reads, 16-byte shared
+// env_kernel_tile_tma<STEP>: env_kernel_tile with the frame phase routed through the TMA unit.
+// A warp assembles a frame in one of its kTmaNbuf shared-memory staging buffers (the same atlas reads, 16-byte shared
 // stores instead of global ones), makes it visible to the async proxy and ONE lane issues a single 9408-byte
 // cp.async.bulk.global.shared::cta for it; the buffer is reused once its bulk group has been read.  The copy engine
 // streams whole frames to HBM while warp 0 is already in the next tile's state phase, and the LSU no longer carries
@@ -96,7 +96,10 @@ __global__ void __launch_bounds__(THREADS, MINB) env_kernel_tile(const EnvParams
 // The copy engine itself is not the problem -- tools/cuda/tma_store_bench.cu streams staged frames at 7.56-7.60 TB/s
 // with as little as ONE 64-thread CTA per SM (per-lane st.global.cs.v4: 7.49) -- but every frame byte now crosses
 // shared memory three times (atlas read, staging write, engine read) instead of once, and the staging buffers
-// (9.4 KB per frame in flight) cost a resident CTA per SM.  Kept selectable (kernel choice 4) with its parity tests.
+// (9.4 KB per frame in flight) cost a resident CTA per SM (profiles/r01_tile_tma_variants.txt).  Kept selectable (kernel
+// choice 4) with its parity tests, in the best shape of the table.
+constexpr int kTmaT = 32, kTmaThreads = 128, kTmaCtas = 3, kTmaNbuf = 1;
+
 __device__ __forceinline__ void bulk_store_frame(uint8_t* gdst, const uint8_t* ssrc) {
   asm volatile("cp.async.bulk.global.shared::cta.bulk_group [%0], [%1], %2;" ::"l"(gdst),
                "r"((uint32_t)__cvta_generic_to_shared(ssrc)), "n"(kImgBytes)
@@ -125,22 +128,20 @@ __device__ __forceinline__ void blit_frame_smem(const uint8_t* atlas_s, const ui
   }
 }
 
-__host__ __device__ constexpr int tile_tma_smem_bytes(int T, int threads, int nbuf) {
-  return tile_smem_bytes(T) + (threads / 32) * nbuf * kImgBytes;
-}
+constexpr int kTmaSmemBytes = tile_smem_bytes(kTmaT) + (kTmaThreads / 32) * kTmaNbuf * kImgBytes;
 
-template <int T, int STEP, int THREADS, int MINB, int NBUF>
-__global__ void __launch_bounds__(THREADS, MINB) env_kernel_tile_tma(const EnvParams p, const int n_tiles) {
+template <int STEP>
+__global__ void __launch_bounds__(kTmaThreads, kTmaCtas) env_kernel_tile_tma(const EnvParams p, const int n_tiles) {
   extern __shared__ __align__(16) uint8_t smem[];
   const int lane = threadIdx.x & 31;
   const int warp = threadIdx.x >> 5;
-  constexpr int warps_per_cta = THREADS / 32;
+  constexpr int warps_per_cta = kTmaThreads / 32;
   const Flags f(p);
   uint8_t* atlas_s = smem;
   uint8_t* kinds_s = smem + kAtlasBytes;
-  uint8_t* sym_s = kinds_s + T * kKindStride;
-  unsigned* mask_s = reinterpret_cast<unsigned*>(smem + tile_smem_bytes(T) - 16);
-  uint8_t* stage_s = smem + tile_smem_bytes(T) + warp * NBUF * kImgBytes;   // this warp's NBUF frame buffers
+  uint8_t* sym_s = kinds_s + kTmaT * kKindStride;
+  unsigned* mask_s = reinterpret_cast<unsigned*>(smem + tile_smem_bytes(kTmaT) - 16);
+  uint8_t* stage_s = smem + tile_smem_bytes(kTmaT) + warp * kTmaNbuf * kImgBytes;   // this warp's kTmaNbuf frame buffers
 
   uint32_t lut[kChunksPerLane];
   if (f.want_rgb) {
@@ -153,9 +154,9 @@ __global__ void __launch_bounds__(THREADS, MINB) env_kernel_tile_tma(const EnvPa
   __syncthreads();
   int tile = s_next;
   while (tile < n_tiles) {
-    const int e0 = tile * T;
+    const int e0 = tile * kTmaT;
     if (warp == 0) {
-      const unsigned m = state_phase<T, STEP>(p, f, e0, lane, kinds_s, sym_s);
+      const unsigned m = state_phase<kTmaT, STEP>(p, f, e0, lane, kinds_s, sym_s);
       if (lane == 0) *mask_s = m;
     } else if (threadIdx.x == 32) {
       s_next = (int)atomicAdd(&p.sched[0], 1u);
@@ -164,18 +165,18 @@ __global__ void __launch_bounds__(THREADS, MINB) env_kernel_tile_tma(const EnvPa
     const unsigned render_mask = *mask_s;
     const int next = s_next;
     if (f.want_sym && render_mask)
-      emit_sym_rows(p.obs_sym + (size_t)e0 * kSymBytes, sym_s, min(T, p.N - e0), render_mask, threadIdx.x, blockDim.x);
+      emit_sym_rows(p.obs_sym + (size_t)e0 * kSymBytes, sym_s, min(kTmaT, p.N - e0), render_mask, threadIdx.x, blockDim.x);
     if (f.want_rgb) {
-      for (int i = warp; i < T; i += warps_per_cta) {
+      for (int i = warp; i < kTmaT; i += warps_per_cta) {
         if (!((render_mask >> i) & 1)) continue;
         uint8_t* stage = stage_s + buf * kImgBytes;
-        if (lane == 0) bulk_wait_read<NBUF - 1>();   // the bulk group that last read this buffer is done with it
+        if (lane == 0) bulk_wait_read<kTmaNbuf - 1>();   // the bulk group that last read this buffer is done with it
         __syncwarp();
         blit_frame_smem(atlas_s, kinds_s + i * kKindStride, lut, stage, lane);
         asm volatile("fence.proxy.async.shared::cta;" ::: "memory");  // generic-proxy writes -> visible to the copy engine
         __syncwarp();
         if (lane == 0) bulk_store_frame(p.obs_rgb + (size_t)(e0 + i) * kImgBytes, stage);
-        buf = (buf + 1 == NBUF) ? 0 : buf + 1;
+        buf = (buf + 1 == kTmaNbuf) ? 0 : buf + 1;
       }
     }
     __syncthreads();
@@ -188,18 +189,15 @@ __global__ void __launch_bounds__(THREADS, MINB) env_kernel_tile_tma(const EnvPa
   }
 }
 
-template <int T, int STEP, bool SWAR, int THREADS = kTileThreads, int MINB = kTileCtasPerSm>
+template <int T, int STEP, bool SWAR>
 static cudaError_t launch_tile_kernel_impl(const EnvParams& p, const LaunchCtx& ctx, cudaStream_t stream) {
   const int n_tiles = (p.N + T - 1) / T;
   const size_t smem = tile_smem_bytes(T);
-  int& blocks_per_sm = ctx.occ[kSlotTile + (T == 8 ? 6 : 0) + (SWAR ? 3 : 0) + STEP];
-  if (!blocks_per_sm) {
-    cudaError_t err = resident_ctas(env_kernel_tile<T, STEP, THREADS, MINB, SWAR>, THREADS, smem, blocks_per_sm);
-    if (err != cudaSuccess) return err;
-    if (MINB < blocks_per_sm) blocks_per_sm = MINB;
-  }
-  const int grid = min(ctx.sm_count * blocks_per_sm, n_tiles);
-  env_kernel_tile<T, STEP, THREADS, MINB, SWAR><<<grid, THREADS, smem, stream>>>(p, n_tiles);
+  int ctas;
+  if (cudaError_t err = resident_ctas(ctx, env_kernel_tile<T, STEP, SWAR>, kTileThreads, smem, ctas, kTileCtasPerSm))
+    return err;
+  const int grid = min(ctx.sm_count * ctas, n_tiles);
+  env_kernel_tile<T, STEP, SWAR><<<grid, kTileThreads, smem, stream>>>(p, n_tiles);
   return cudaGetLastError();
 }
 template <int T, int STEP>
@@ -208,27 +206,16 @@ static cudaError_t launch_tile_kernel_step(const EnvParams& p, const LaunchCtx& 
                                 : launch_tile_kernel_impl<T, STEP, false>(p, ctx, stream);
 }
 
-#ifndef MERLIN_TMA_T
-#define MERLIN_TMA_T 32
-#define MERLIN_TMA_THREADS 128
-#define MERLIN_TMA_CTAS 3
-#define MERLIN_TMA_NBUF 1
-#endif
-template <int T, int STEP, int THREADS = MERLIN_TMA_THREADS, int MINB = MERLIN_TMA_CTAS, int NBUF = MERLIN_TMA_NBUF>
+template <int STEP>
 static cudaError_t launch_tile_tma_kernel_step(const EnvParams& p, const LaunchCtx& ctx, cudaStream_t stream) {
-  const int n_tiles = (p.N + T - 1) / T;
-  const size_t smem = tile_tma_smem_bytes(T, THREADS, NBUF);
-  int& blocks_per_sm = ctx.occ[kSlotTma + STEP];
-  if (!blocks_per_sm) {
-    cudaError_t err = resident_ctas(env_kernel_tile_tma<T, STEP, THREADS, MINB, NBUF>, THREADS, smem, blocks_per_sm);
-    if (err != cudaSuccess) return err;
-    if (MINB < blocks_per_sm) blocks_per_sm = MINB;
-  }
-  const int grid = min(ctx.sm_count * blocks_per_sm, n_tiles);
-  env_kernel_tile_tma<T, STEP, THREADS, MINB, NBUF><<<grid, THREADS, smem, stream>>>(p, n_tiles);
+  const int n_tiles = (p.N + kTmaT - 1) / kTmaT;
+  int ctas;
+  if (cudaError_t err = resident_ctas(ctx, env_kernel_tile_tma<STEP>, kTmaThreads, kTmaSmemBytes, ctas, kTmaCtas))
+    return err;
+  const int grid = min(ctx.sm_count * ctas, n_tiles);
+  env_kernel_tile_tma<STEP><<<grid, kTmaThreads, kTmaSmemBytes, stream>>>(p, n_tiles);
   return cudaGetLastError();
 }
-
 
 cudaError_t launch_tile_kernel(int T, int step, const EnvParams& p, const LaunchCtx& ctx, cudaStream_t stream) {
   if (T == 16) {
@@ -241,9 +228,9 @@ cudaError_t launch_tile_kernel(int T, int step, const EnvParams& p, const Launch
   return launch_tile_kernel_step<8, 2>(p, ctx, stream);
 }
 cudaError_t launch_tile_tma_kernel(int step, const EnvParams& p, const LaunchCtx& ctx, cudaStream_t stream) {
-  if (step == 0) return launch_tile_tma_kernel_step<MERLIN_TMA_T, 0>(p, ctx, stream);
-  if (step == 1) return launch_tile_tma_kernel_step<MERLIN_TMA_T, 1>(p, ctx, stream);
-  return launch_tile_tma_kernel_step<MERLIN_TMA_T, 2>(p, ctx, stream);
+  if (step == 0) return launch_tile_tma_kernel_step<0>(p, ctx, stream);
+  if (step == 1) return launch_tile_tma_kernel_step<1>(p, ctx, stream);
+  return launch_tile_tma_kernel_step<2>(p, ctx, stream);
 }
 
 }  // namespace merlin

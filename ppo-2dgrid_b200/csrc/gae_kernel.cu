@@ -20,10 +20,6 @@
 
 namespace merlin {
 
-#ifndef MERLIN_GAE_CHUNK_SMALL
-#define MERLIN_GAE_CHUNK_SMALL 32
-#define MERLIN_GAE_CHUNK_LARGE 16
-#endif
 template <int kChunk>
 __global__ void __launch_bounds__(128) gae_kernel(const float* __restrict__ rew, const float* __restrict__ val,
                                                   const float* __restrict__ done, const float* __restrict__ last_val,
@@ -37,9 +33,10 @@ __global__ void __launch_bounds__(128) gae_kernel(const float* __restrict__ rew,
   // The recurrence is serial in t but its loads are not: fetch kChunk time steps (3 x kChunk independent, coalesced
   // loads in flight per thread) before running the kChunk dependent updates, so a short rollout (a few thousand envs,
   // one warp per SM) is bound by the arithmetic chain rather than by kChunk-times-fewer memory round trips.
-  // Measured on B200 (tools/gae_variants.sh): kChunk = 32 for small rollouts (T=128 x N=4096: 14.3 us vs 20.5 with 8
-  // -- 4 memory round trips per thread instead of 16; 149 registers do not matter at one warp per SM), 16 for
-  // rollouts that fill the machine (T=64 x N=1M: 0.90 of the HBM copy peak vs 0.885 with 8 and 0.87 with 4).
+  // Measured on B200 (profiles/r01_gae_chunk_variants.txt): kChunk = 32 for small rollouts (kGaeChunkSmall; T=128 x
+  // N=4096: 14.3 us vs 20.5 with 8 -- 4 memory round trips per thread instead of 16; 149 registers do not matter at one
+  // warp per SM), 16 for rollouts that fill the machine (kGaeChunkLarge; T=64 x N=1M: 0.90 of the HBM copy peak vs 0.885
+  // with 8 and 0.87 with 4).
   int t = T - 1;
   for (; t >= kChunk - 1; t -= kChunk) {
     float r[kChunk], v[kChunk], d[kChunk];
@@ -148,15 +145,13 @@ __global__ void __launch_bounds__(256) gae_tile_kernel(const float* __restrict__
 // Where the tile kernel runs.  32 calls replayed from a CUDA graph, L2-warm (tools/bench_gae.py, T = 128), tile kernel vs
 // one thread per env: 6.06 vs 5.61 us at 32 envs (one CTA: nothing to spread), 6.06 vs 7.57 at 1024, 6.14 vs 7.61 at 4096,
 // 12.2 vs 11.8 at 16 384 (512 CTAs of 48 KB: four rounds per SM).
-#ifndef MERLIN_GAE_TILE_MAX_ENVS
-#define MERLIN_GAE_TILE_MIN_ENVS 128
-#define MERLIN_GAE_TILE_MAX_ENVS 8192
-#endif
+constexpr int kGaeTileMinEnvs = 128, kGaeTileMaxEnvs = 8192;
+constexpr int kGaeChunkSmall = 32, kGaeChunkLarge = 16;   // see gae_kernel
 
 cudaError_t launch_gae(const float* rew, const float* val, const float* done, const float* last_val, float* adv,
                        float* ret, int T, int N, double gamma, double lam, cudaStream_t stream) {
   // small rollouts: 32-thread blocks spread the envs over more SMs (4096 envs -> 128 blocks instead of 32)
-  if (N >= MERLIN_GAE_TILE_MIN_ENVS && N <= MERLIN_GAE_TILE_MAX_ENVS) {
+  if (N >= kGaeTileMinEnvs && N <= kGaeTileMaxEnvs) {
     gae_tile_kernel<<<(N + 31) / 32, 256, 0, stream>>>(rew, val, done, last_val, adv, ret, T, N, gamma, (float)gamma,
                                                        (float)(gamma * lam));
     return cudaGetLastError();
@@ -165,11 +160,11 @@ cudaError_t launch_gae(const float* rew, const float* val, const float* done, co
   const int threads = N >= 128 * 148 * 4 ? 128 : 32;
   const int blocks = (N + threads - 1) / threads;
   if (large)
-    gae_kernel<MERLIN_GAE_CHUNK_LARGE><<<blocks, threads, 0, stream>>>(rew, val, done, last_val, adv, ret, T, N, gamma,
-                                                                       (float)gamma, (float)(gamma * lam));
+    gae_kernel<kGaeChunkLarge><<<blocks, threads, 0, stream>>>(rew, val, done, last_val, adv, ret, T, N, gamma,
+                                                               (float)gamma, (float)(gamma * lam));
   else
-    gae_kernel<MERLIN_GAE_CHUNK_SMALL><<<blocks, threads, 0, stream>>>(rew, val, done, last_val, adv, ret, T, N, gamma,
-                                                                       (float)gamma, (float)(gamma * lam));
+    gae_kernel<kGaeChunkSmall><<<blocks, threads, 0, stream>>>(rew, val, done, last_val, adv, ret, T, N, gamma,
+                                                               (float)gamma, (float)(gamma * lam));
   return cudaGetLastError();
 }
 

@@ -99,15 +99,13 @@ __global__ void __launch_bounds__(256, 2) render_kernel(const RenderParams p) {
   }
 }
 
-#ifndef MERLIN_RENDER_GROUP32_MIN_FRAMES
-#define MERLIN_RENDER_GROUP32_MIN_FRAMES 65536
-#endif
+constexpr int kRenderGroup32MinFrames = 65536;
 cudaError_t launch_render(const RenderParams& p, bool blocked, int sm_count, cudaStream_t stream) {
   if (p.M <= 0) return cudaSuccess;
   constexpr int threads = 256, warps = threads / 32;
   const size_t smem = kAtlasBytes + warps * kWarpKindStride;
   RenderParams q = p;
-  q.group_frames = p.M >= MERLIN_RENDER_GROUP32_MIN_FRAMES ? 32 : warps;
+  q.group_frames = p.M >= kRenderGroup32MinFrames ? 32 : warps;
   const int grid = min(sm_count * 2, (p.M + q.group_frames - 1) / q.group_frames);
   if (blocked) render_kernel<true><<<grid, threads, smem, stream>>>(q);
   else render_kernel<false><<<grid, threads, smem, stream>>>(q);
@@ -129,9 +127,7 @@ constexpr int kF32Chunks = kImgBytes / 4;                  // 2352 float4 chunks
 constexpr int kF32Iters = (kF32Chunks + 31) / 32;          // 74
 constexpr int kRenderF32Group = 8;                          // frames per ticket: 301 KB, like the u8 kernels' groups
 constexpr int kRenderF32Threads = 256;
-#ifndef MERLIN_RENDER_F32_CTA_FRAMES_MAX
-#define MERLIN_RENDER_F32_CTA_FRAMES_MAX 8192
-#endif
+constexpr int kRenderF32CtaFramesMax = 8192;
 
 __host__ __device__ constexpr size_t render_f32_smem(int cap_tiles) {
   return (size_t)cap_tiles * kTileBytes * 4 + 128 + 592 * 2 + (kRenderF32Threads / 32) * 128;
@@ -256,7 +252,7 @@ cudaError_t launch_render_f32(const RenderParams& p, int sm_count, cudaStream_t 
   // over the frames (no ticket counter involved).  With a warp per frame, 4096 frames are 1.15 rounds of the 3552 resident
   // warps, i.e. two rounds of which the second is 15 % full; with a CTA per frame they are 9.2 rounds of 444 CTAs, i.e. ten.
   // Above: groups of 8 frames per ticket, one warp per frame.
-  q.frame_per_cta = p.M <= MERLIN_RENDER_F32_CTA_FRAMES_MAX ? 1 : 0;
+  q.frame_per_cta = p.M <= kRenderF32CtaFramesMax ? 1 : 0;
   const int grid = q.frame_per_cta ? min(p.M, sm_count * per_sm)
                                    : min(sm_count * per_sm, (p.M + kRenderF32Group - 1) / kRenderF32Group);
   render_f32_kernel<<<grid, kRenderF32Threads, smem, stream>>>(q);
