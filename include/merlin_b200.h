@@ -10,6 +10,8 @@
  *   merlin_env_upload_layouts     the result of MiniGridEnv.reset() -> _gen_grid()
  *                                 src/custom_envs/medium_hard_env.py:12-45 (and the four siblings)
  *   merlin_env_generate_layouts   the same `_gen_grid` routines run on the device (fresh layouts without a host pool)
+ *   merlin_env_generate_seeded_layouts   env.reset(seed=s) -> _gen_grid() for a list of seeds, on the device: the
+ *                                 `_gen_grid` routines fed by numpy's default_rng(s) stream, restated
  *   merlin_env_set_tile_atlas     Grid.render_tile cache used by RGBImgPartialObsWrapper
  *                                 (src/scenario_creator/scenario_creator.py:48, tile_size 8)
  *   merlin_env_reset              env.reset()   src/ppo.py:35,65,96 ; src/fomaml.py:63,92,184
@@ -116,8 +118,9 @@ int merlin_env_upload_layouts(merlin_env_t* h, const uint8_t* cells, const int32
 /* Generate the pool ON THE DEVICE: n_layouts layouts of `difficulty` (the reference's `_gen_grid` routines,
  * src/custom_envs/{easy,medium,medium_hard,hard,hardest}_env.py, same algorithm and distributions) from a counter-based
  * generator keyed by (seed, first_number + slot).  NOT the layouts numpy's PCG64 stream would give for a reference seed:
- * use merlin_env_upload_layouts with host-generated layouts to reproduce `env.reset(seed=s)`.  Replaces the pool (in
- * place when n_layouts is unchanged), resets the cursors.  Synchronous. */
+ * use merlin_env_generate_seeded_layouts (or merlin_env_upload_layouts with host-generated layouts) to reproduce
+ * `env.reset(seed=s)`.  Replaces the pool (in place when n_layouts is unchanged), resets the cursors.  Synchronous.
+ * Sides below 6 (easy), 8 (hardest) or 4 (the others) are rejected. */
 #define MERLIN_D_EASY 0
 #define MERLIN_D_MEDIUM 1
 #define MERLIN_D_MEDIUMHARD 2
@@ -125,6 +128,21 @@ int merlin_env_upload_layouts(merlin_env_t* h, const uint8_t* cells, const int32
 #define MERLIN_D_HARDEST 4
 int merlin_env_generate_layouts(merlin_env_t* h, int32_t difficulty, uint64_t seed, int64_t first_number,
                                 int32_t n_layouts, void* stream);
+/* Generate the pool ON THE DEVICE from reference seeds: slot i gets the layout of `env.reset(seed=seeds[i])` -> `_gen_grid`
+ * (src/custom_envs/{easy,medium,medium_hard,hard,hardest}_env.py), byte for byte the layout the reference and
+ * merlin_b200.layouts.generate build.  The routines are those of merlin_env_generate_layouts, fed by a restatement of
+ * numpy's `default_rng(seed)`: SeedSequence -> PCG64 (XSL-RR), `Generator.integers` (Lemire's bounded method on the
+ * buffered next_uint32) and `Generator.choice(replace=False)` (Floyd's algorithm + shuffle), pinned to numpy 2.3.5.
+ * seeds: HOST u64[n_layouts].  Same pool semantics as merlin_env_generate_layouts: replaced in place when n_layouts is
+ * unchanged (CUDA graphs captured over reset/step stay valid), cursors reset, the same atlas mask.  Synchronous.
+ * Rejects what merlin_env_generate_layouts rejects, and hard below 5.
+ * Where the reference's routine raises or never returns for a seed (a `place_obj` that exhausts max_tries=100, or 2^20
+ * tries for max_tries=inf; `integers` or `choice` on an empty range), returns MERLIN_EINVAL and merlin_last_error()
+ * names the first such seed.  The pool then holds the layouts of the other seeds and garbage in the failed slots:
+ * reset() and set_cursors() fail with MERLIN_ESTATE (so does step(), which needs a reset) until the next successful
+ * upload or generation; read_layouts() still works.  Graphs captured earlier are not stopped: do not replay them. */
+int merlin_env_generate_seeded_layouts(merlin_env_t* h, int32_t difficulty, const uint64_t* seeds, int32_t n_layouts,
+                                       void* stream);
 /* Synchronous copy of the current pool to HOST buffers (either may be NULL): cells u8[n_layouts][H*W], agent_xyd
  * i32[n_layouts][3]; merlin_env_layout_count gives n_layouts. */
 int merlin_env_read_layouts(merlin_env_t* h, uint8_t* cells, int32_t* agent_xyd);

@@ -60,6 +60,7 @@ struct merlin_env {
   bool has_atlas = false;
   int n_present = kAtlasTiles;           // atlas slots the current layout pool can show (host copy of the popcount)
   bool was_reset = false;
+  bool pool_failed = false;              // the last seeded generation hit a seed it could not build: no reset until a new pool
   int64_t launches = 0;
   // per-handle tuning knobs (-1 = follow the process-wide default) and occupancy cache
   int kernel_choice = -1;
@@ -154,6 +155,54 @@ static int launch_failed(merlin_env* h, cudaError_t err, const char* what, void*
   cudaMemsetAsync(h->sched, 0, kSchedWords * sizeof(unsigned), static_cast<cudaStream_t>(stream));
   cudaGetLastError();
   return cuda_fail(err, what);
+}
+
+// Storage for a pool of n_layouts.  A pool of another size gets new storage; an equal-sized pool is overwritten in
+// place, so device pointers (and CUDA graphs captured over them) stay valid across uploads and generations.
+static int pool_storage(merlin_env* h, int n_layouts) {
+  if (n_layouts == h->n_layouts) return MERLIN_OK;
+  uint8_t* d_cells = nullptr;
+  uint32_t* d_agent = nullptr;
+  if (cudaMalloc(&d_cells, (size_t)n_layouts * h->cell_stride) != cudaSuccess ||
+      cudaMalloc(&d_agent, (size_t)n_layouts * sizeof(uint32_t)) != cudaSuccess) {
+    cudaFree(d_cells);
+    return cuda_fail(cudaGetLastError(), "layout pool allocation");
+  }
+  cudaFree(h->pool_cells); cudaFree(h->pool_agent);
+  h->pool_cells = d_cells; h->pool_agent = d_agent; h->n_layouts = n_layouts;
+  return MERLIN_OK;
+}
+
+// Arguments of the two device generators.  The seeded one also rejects hard below 5 (its routine raises or never
+// returns there for some seeds; the other generator treats such draws as failed attempts).
+static int check_generation(merlin_env* h, int difficulty, int n_layouts, bool seeded) {
+  if (!h) return fail(MERLIN_EINVAL, "null handle");
+  if (difficulty < MERLIN_D_EASY || difficulty > MERLIN_D_HARDEST) return fail(MERLIN_EINVAL, "unknown difficulty id");
+  if (n_layouts < 1)
+    return fail(MERLIN_EINVAL, seeded ? "merlin_env_generate_seeded_layouts: no seeds"
+                                      : "merlin_env_generate_layouts: bad count / first_number");
+  const int W = h->cfg.width, H = h->cfg.height;
+  int min_side = difficulty == MERLIN_D_HARDEST ? 8 : (difficulty == MERLIN_D_EASY ? 6 : 4);
+  if (seeded && difficulty == MERLIN_D_HARD) min_side = 5;
+  if (W < min_side || H < min_side) return fail(MERLIN_EINVAL, "grid too small for this difficulty's layout routine");
+  return MERLIN_OK;
+}
+
+// The shared tail of a device generation that built every slot: the atlas slots a generated pool can show (the
+// invisible tile, highlighted empty, the agent, wall and goal), the cursors reset; reset() must follow.
+static int generated_pool_ready(merlin_env* h) {
+  uint32_t present[4] = {(1u << KIND_UNSEEN) | (1u << CODE_EMPTY) | (1u << KIND_AGENT), 0, 0, 0};
+  const uint32_t goal = T_GOAL | (1u << 4);
+  present[CODE_WALL >> 5] |= 1u << (CODE_WALL & 31);
+  present[goal >> 5] |= 1u << (goal & 31);
+  if (h->mutable_grid) present[0] = present[1] = present[2] = present[3] = 0xffffffffu;
+  const cudaError_t err = cudaMemcpy(h->tile_present, present, sizeof present, cudaMemcpyHostToDevice);
+  if (err != cudaSuccess) return cuda_fail(err, "layout generation (mask)");
+  h->n_present = count_present(present);
+  h->launches += 1;
+  h->was_reset = false;
+  h->pool_failed = false;
+  return merlin_env_set_cursors(h, nullptr);
 }
 
 extern "C" {
@@ -300,66 +349,72 @@ int merlin_env_upload_layouts(merlin_env_t* h, const uint8_t* cells, const int32
   if (h->mutable_grid) present[0] = present[1] = present[2] = present[3] = 0xffffffffu;
   cudaError_t err = cudaDeviceSynchronize();  // nothing may still be reading the old pool
   if (err != cudaSuccess) return cuda_fail(err, "layout upload (sync)");
-  if (n_layouts != h->n_layouts) {
-    // a pool of another size gets new storage; an equal-sized pool is overwritten in place, so device pointers (and
-    // CUDA graphs captured over them) stay valid across uploads
-    uint8_t* d_cells = nullptr;
-    uint32_t* d_agent = nullptr;
-    if (cudaMalloc(&d_cells, packed.size()) != cudaSuccess || cudaMalloc(&d_agent, agent.size() * sizeof(uint32_t)) != cudaSuccess) {
-      cudaFree(d_cells);
-      return cuda_fail(cudaGetLastError(), "layout pool allocation");
-    }
-    cudaFree(h->pool_cells); cudaFree(h->pool_agent);
-    h->pool_cells = d_cells; h->pool_agent = d_agent; h->n_layouts = n_layouts;
-  }
+  if (const int rc = pool_storage(h, n_layouts)) return rc;
   err = cudaMemcpy(h->pool_cells, packed.data(), packed.size(), cudaMemcpyHostToDevice);
   if (err == cudaSuccess) err = cudaMemcpy(h->pool_agent, agent.data(), agent.size() * sizeof(uint32_t), cudaMemcpyHostToDevice);
   if (err == cudaSuccess) err = cudaMemcpy(h->tile_present, present, sizeof present, cudaMemcpyHostToDevice);
   if (err != cudaSuccess) return cuda_fail(err, "layout upload");
   h->n_present = count_present(present);
   h->was_reset = false;
+  h->pool_failed = false;
   cudaMemset(h->sched, 0, kSchedWords * sizeof(unsigned));  // the device is idle here: a cheap place to rearm the tickets
   return merlin_env_set_cursors(h, nullptr);
 }
 
 int merlin_env_generate_layouts(merlin_env_t* h, int32_t difficulty, uint64_t seed, int64_t first_number,
                                 int32_t n_layouts, void* stream) {
-  if (!h) return fail(MERLIN_EINVAL, "null handle");
-  if (difficulty < MERLIN_D_EASY || difficulty > MERLIN_D_HARDEST) return fail(MERLIN_EINVAL, "unknown difficulty id");
-  if (n_layouts < 1 || first_number < 0) return fail(MERLIN_EINVAL, "merlin_env_generate_layouts: bad count / first_number");
-  const int W = h->cfg.width, H = h->cfg.height;
-  const int min_side = difficulty == MERLIN_D_HARDEST ? 8 : (difficulty == MERLIN_D_EASY ? 6 : 4);
-  if (W < min_side || H < min_side) return fail(MERLIN_EINVAL, "grid too small for this difficulty's layout routine");
+  if (const int rc = check_generation(h, difficulty, n_layouts, false)) return rc;
+  if (first_number < 0) return fail(MERLIN_EINVAL, "merlin_env_generate_layouts: bad count / first_number");
   DeviceGuard guard(h->cfg.device);
   cudaError_t err = cudaDeviceSynchronize();  // nothing may still be reading the old pool
   if (err != cudaSuccess) return cuda_fail(err, "layout generation (sync)");
-  if (n_layouts != h->n_layouts) {
-    uint8_t* d_cells = nullptr;
-    uint32_t* d_agent = nullptr;
-    if (cudaMalloc(&d_cells, (size_t)n_layouts * h->cell_stride) != cudaSuccess ||
-        cudaMalloc(&d_agent, (size_t)n_layouts * sizeof(uint32_t)) != cudaSuccess) {
-      cudaFree(d_cells);
-      return cuda_fail(cudaGetLastError(), "layout pool allocation");
-    }
-    cudaFree(h->pool_cells); cudaFree(h->pool_agent);
-    h->pool_cells = d_cells; h->pool_agent = d_agent; h->n_layouts = n_layouts;
-  }
+  if (const int rc = pool_storage(h, n_layouts)) return rc;
   cudaStream_t s = static_cast<cudaStream_t>(stream);
-  err = launch_layouts(h->pool_cells, h->pool_agent, h->cell_stride, W, H, difficulty, seed, first_number, 0, n_layouts,
-                       h->sm_count, s);
+  err = launch_layouts(h->pool_cells, h->pool_agent, h->cell_stride, h->cfg.width, h->cfg.height, difficulty, seed,
+                       first_number, 0, n_layouts, h->sm_count, s);
   if (err == cudaSuccess) err = cudaStreamSynchronize(s);
   if (err != cudaSuccess) return cuda_fail(err, "layout generation");
-  uint32_t present[4] = {(1u << KIND_UNSEEN) | (1u << CODE_EMPTY) | (1u << KIND_AGENT), 0, 0, 0};
-  const uint32_t goal = T_GOAL | (1u << 4);
-  present[CODE_WALL >> 5] |= 1u << (CODE_WALL & 31);
-  present[goal >> 5] |= 1u << (goal & 31);
-  if (h->mutable_grid) present[0] = present[1] = present[2] = present[3] = 0xffffffffu;
-  err = cudaMemcpy(h->tile_present, present, sizeof present, cudaMemcpyHostToDevice);
-  if (err != cudaSuccess) return cuda_fail(err, "layout generation (mask)");
-  h->n_present = count_present(present);
-  h->launches += 1;
+  return generated_pool_ready(h);
+}
+
+int merlin_env_generate_seeded_layouts(merlin_env_t* h, int32_t difficulty, const uint64_t* seeds, int32_t n_layouts,
+                                       void* stream) {
+  if (h && !seeds) return fail(MERLIN_EINVAL, "merlin_env_generate_seeded_layouts: null seeds");
+  if (const int rc = check_generation(h, difficulty, n_layouts, true)) return rc;
+  DeviceGuard guard(h->cfg.device);
+  cudaError_t err = cudaDeviceSynchronize();  // nothing may still be reading the old pool
+  if (err != cudaSuccess) return cuda_fail(err, "seeded layout generation (sync)");
+  if (const int rc = pool_storage(h, n_layouts)) return rc;
+  // from here on the pool is being rewritten: it counts as failed until the kernel has built every slot
+  h->pool_failed = true;
   h->was_reset = false;
-  return merlin_env_set_cursors(h, nullptr);
+  cudaStream_t s = static_cast<cudaStream_t>(stream);
+  uint64_t* d_seeds = nullptr;
+  int* d_first_failed = nullptr;
+  int first_failed = n_layouts;
+  if (cudaMalloc(&d_seeds, (size_t)n_layouts * sizeof(uint64_t)) != cudaSuccess ||
+      cudaMalloc(&d_first_failed, sizeof(int)) != cudaSuccess) {
+    cudaFree(d_seeds);
+    return cuda_fail(cudaGetLastError(), "seeded layout generation (allocation)");
+  }
+  err = cudaMemcpyAsync(d_seeds, seeds, (size_t)n_layouts * sizeof(uint64_t), cudaMemcpyHostToDevice, s);
+  if (err == cudaSuccess) err = cudaMemcpyAsync(d_first_failed, &first_failed, sizeof(int), cudaMemcpyHostToDevice, s);
+  if (err == cudaSuccess)
+    err = launch_seeded_layouts(h->pool_cells, h->pool_agent, h->cell_stride, h->cfg.width, h->cfg.height, difficulty,
+                                d_seeds, n_layouts, d_first_failed, h->sm_count, s);
+  if (err == cudaSuccess) err = cudaMemcpyAsync(&first_failed, d_first_failed, sizeof(int), cudaMemcpyDeviceToHost, s);
+  if (err == cudaSuccess) err = cudaStreamSynchronize(s);
+  cudaFree(d_seeds); cudaFree(d_first_failed);
+  if (err != cudaSuccess) return cuda_fail(err, "seeded layout generation");
+  if (first_failed < n_layouts) {
+    static const char* const kNames[] = {"easy", "medium", "mediumhard", "hard", "hardest"};
+    char msg[224];
+    std::snprintf(msg, sizeof msg, "seed %llu (slot %d): the %s %dx%d layout routine raises or never returns for it; "
+                  "the pool is incomplete until the next upload or generation",
+                  (unsigned long long)seeds[first_failed], first_failed, kNames[difficulty], h->cfg.width, h->cfg.height);
+    return fail(MERLIN_EINVAL, msg);
+  }
+  return generated_pool_ready(h);
 }
 
 int merlin_env_read_layouts(merlin_env_t* h, uint8_t* cells, int32_t* agent_xyd) {
@@ -404,6 +459,7 @@ int merlin_env_set_tile_atlas(merlin_env_t* h, const uint8_t* tiles, int32_t n_t
 int merlin_env_set_cursors(merlin_env_t* h, const int32_t* cursor) {
   if (!h) return fail(MERLIN_EINVAL, "null handle");
   if (h->n_layouts < 1) return fail(MERLIN_ESTATE, "upload layouts first");
+  if (h->pool_failed) return fail(MERLIN_ESTATE, "the layout pool is incomplete: the last seeded generation failed");
   const int N = h->cfg.n_envs;
   std::vector<int4> st((size_t)N);
   for (int e = 0; e < N; ++e) {
@@ -421,6 +477,7 @@ int merlin_env_set_cursors(merlin_env_t* h, const int32_t* cursor) {
 int merlin_env_reset(merlin_env_t* h, const uint8_t* mask, uint8_t* obs_rgb, uint8_t* obs_sym, void* stream) {
   if (!h) return fail(MERLIN_EINVAL, "null handle");
   if (h->n_layouts < 1) return fail(MERLIN_ESTATE, "reset before layouts were uploaded");
+  if (h->pool_failed) return fail(MERLIN_ESTATE, "the layout pool is incomplete: the last seeded generation failed");
   if (obs_rgb && !h->has_atlas) return fail(MERLIN_ESTATE, "RGB observation requested before the tile atlas was set");
   if (mask && !h->was_reset) return fail(MERLIN_ESTATE, "the first reset must cover every env (mask = NULL)");
   if (obs_rgb && (reinterpret_cast<uintptr_t>(obs_rgb) & 15)) return fail(MERLIN_EINVAL, "obs_rgb must be 16-byte aligned");

@@ -146,6 +146,11 @@ cudaError_t launch_render_f32(const RenderParams& p, int sm_count, cudaStream_t 
 cudaError_t launch_layouts(uint8_t* pool_cells, uint32_t* pool_agent, int cell_stride, int W, int H, int difficulty,
                            uint64_t seed, long long first_number, int first_slot, int count, int sm_count,
                            cudaStream_t stream);
+// slot i <- the layout of `env.reset(seed=seeds[i])` (numpy's stream, np_random.cuh); seeds: DEVICE u64[count];
+// *first_failed (DEVICE, preset to count) <- the smallest slot whose seed the host generator could not build
+cudaError_t launch_seeded_layouts(uint8_t* pool_cells, uint32_t* pool_agent, int cell_stride, int W, int H,
+                                  int difficulty, const uint64_t* seeds, int count, int* first_failed, int sm_count,
+                                  cudaStream_t stream);
 // FullyObsWrapper.observation for every env: Grid.encode() of the current grid, u8[N][W][H][3] indexed [x][y][c],
 // with the agent's cell replaced by (OBJECT_TO_IDX["agent"] = 10, COLOR_TO_IDX["red"] = 0, agent_dir).
 cudaError_t launch_full_obs(const EnvParams& p, uint8_t* out, int sm_count, cudaStream_t stream);

@@ -17,8 +17,8 @@ F_AUTO_RESET, F_RESET_SAME, F_SEVEN_ACTIONS, F_STUCK_PENALTY, F_EXPLORE_BONUS = 
 
 EXPORTS = (
     "merlin_env_default_config", "merlin_env_create", "merlin_env_destroy", "merlin_env_upload_layouts",
-    "merlin_env_generate_layouts", "merlin_env_read_layouts", "merlin_env_layout_count",
-    "merlin_env_set_tile_atlas", "merlin_env_set_cursors", "merlin_env_reset", "merlin_env_step",
+    "merlin_env_generate_layouts", "merlin_env_generate_seeded_layouts", "merlin_env_read_layouts",
+    "merlin_env_layout_count", "merlin_env_set_tile_atlas", "merlin_env_set_cursors", "merlin_env_reset", "merlin_env_step",
     "merlin_env_state_ptrs", "merlin_env_read_state", "merlin_env_bad_actions", "merlin_env_launch_count",
     "merlin_set_kernel_choice", "merlin_set_observation_path", "merlin_env_step_kernel", "merlin_env_render", "merlin_env_render_f32", "merlin_env_full_obs", "merlin_gae",
     "merlin_pack_cell", "merlin_last_error", "merlin_version",
@@ -67,6 +67,7 @@ def load():
     lib.merlin_env_destroy.argtypes = [vp]
     lib.merlin_env_upload_layouts.argtypes = [vp, vp, vp, i32]
     lib.merlin_env_generate_layouts.argtypes = [vp, i32, C.c_uint64, i64, i32, vp]
+    lib.merlin_env_generate_seeded_layouts.argtypes = [vp, i32, vp, i32, vp]
     lib.merlin_env_read_layouts.argtypes = [vp, vp, vp]
     lib.merlin_env_layout_count.argtypes = [vp]
     lib.merlin_env_set_tile_atlas.argtypes = [vp, vp, i32]
@@ -103,7 +104,7 @@ def load():
     lib.merlin_last_error.restype = C.c_char_p
     lib.merlin_version.restype = C.c_char_p
     for name in ("merlin_env_create", "merlin_env_destroy", "merlin_env_upload_layouts", "merlin_env_set_tile_atlas",
-                 "merlin_env_generate_layouts", "merlin_env_read_layouts", "merlin_env_layout_count",
+                 "merlin_env_generate_layouts", "merlin_env_generate_seeded_layouts", "merlin_env_read_layouts", "merlin_env_layout_count",
                  "merlin_env_set_cursors", "merlin_env_reset", "merlin_env_step", "merlin_env_state_ptrs",
                  "merlin_env_read_state", "merlin_env_bad_actions", "merlin_gae", "merlin_env_policy_step",
                  "merlin_env_seed_sampler", "merlin_env_rearm", "merlin_env_set_kernel_choice",

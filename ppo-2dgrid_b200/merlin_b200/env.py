@@ -10,6 +10,7 @@ tensors and forwards pointers through the C ABI (include/merlin_b200.h).
 from __future__ import annotations
 
 import ctypes as C
+import operator
 
 import numpy as np
 import torch
@@ -57,9 +58,12 @@ class BatchedMerlinEnv:
     def __init__(self, num_envs, cells=None, agent=None, *, enc=None, width=None, height=None, max_steps=None,
                  device="cuda", n_actions=3, auto_reset=True, reset_mode="next", stuck_penalty=False,
                  stuck_max_stay=3, stuck_penalty_value=-0.1, exploration_bonus=0.0, want_symbolic=True,
-                 want_rgb=True, generate=None, episode_stats=True):
+                 want_rgb=True, generate=None, generate_seeded=None, episode_stats=True):
         """cells: packed u8[L, H*W] (merlin_b200.codes) or `enc`: Grid.encode() arrays u8[L, W, H, 3];
-        agent: i32[L, 3] = (x, y, dir).  `reset_mode`: "next" advances each env's pool cursor by num_envs at
+        agent: i32[L, 3] = (x, y, dir).  Instead of a pool: `generate=(difficulty, seed, n_layouts)` generates one on
+        the device (`generate_layouts`), `generate_seeded=(difficulty, seeds)` the reference's layouts of `seeds` on the
+        device (`generate_seeded_layouts`); both need width/height.
+        `reset_mode`: "next" advances each env's pool cursor by num_envs at
         every restart, modulo the pool size (by one slot when the pool size divides num_envs) (PPO: a fresh layout per episode), "same" replays the same layout (FOMAML task)."""
         self.device = torch.device(device)
         if self.device.type != "cuda" or not torch.cuda.is_available():
@@ -74,11 +78,15 @@ class BatchedMerlinEnv:
             enc = np.asarray(enc)
             width, height = enc.shape[1], enc.shape[2]
             cells = codes.pack_encoding(enc)
-        if generate is not None:
+        if generate is not None and generate_seeded is not None:
+            raise ValueError("generate and generate_seeded are exclusive")
+        if generate is not None or generate_seeded is not None:
             if width is None:
-                raise ValueError("width/height are required with generate=(difficulty, seed, n_layouts)")
+                raise ValueError("width/height are required with generate=(difficulty, seed, n_layouts) or "
+                                 "generate_seeded=(difficulty, seeds)")
         elif cells is None or agent is None:
-            raise ValueError("a layout pool (cells or enc, and agent) or generate=(difficulty, seed, n_layouts) is required")
+            raise ValueError("a layout pool (cells or enc, and agent), generate=(difficulty, seed, n_layouts) or "
+                             "generate_seeded=(difficulty, seeds) is required")
         else:
             cells = np.ascontiguousarray(cells, dtype=np.uint8)
             if width is None:
@@ -86,7 +94,7 @@ class BatchedMerlinEnv:
         self.num_envs, self.width, self.height = int(num_envs), int(width), int(height)
         # what evaluators need to rebuild this env's layouts for other seeds: the layout routine (known when the pool was
         # generated here or the env came from ScenarioCreator.create_batched_env, else None) and the grid size
-        self.difficulty = generate[0] if generate is not None else None
+        self.difficulty = next((g[0] for g in (generate, generate_seeded) if g is not None), None)
         self.size = self.width
         self.n_actions = n_actions
         self.want_symbolic, self.want_rgb = want_symbolic, want_rgb
@@ -119,6 +127,8 @@ class BatchedMerlinEnv:
         _lib.check(self._lib.merlin_env_set_tile_atlas(self._h, atlas.ctypes.data, atlas.shape[0]))
         if generate is not None:
             self.generate_layouts(*generate)
+        elif generate_seeded is not None:
+            self.generate_seeded_layouts(*generate_seeded)
         else:
             self.upload_layouts(cells, agent)
 
@@ -171,6 +181,33 @@ class BatchedMerlinEnv:
                                                          int(first_number), int(n_layouts), self._stream()))
         self.n_layouts = int(n_layouts)
         self._pool_cells_host = None
+
+    def generate_seeded_layouts(self, difficulty, seeds):
+        """Fill the pool on the device with the layouts of `env.reset(seed=s)` for every s in `seeds` (Python ints in
+        [0, 2^64)): byte for byte what `merlin_b200.layouts.generate(difficulty, size, seeds)` builds on the host.
+        Resets the cursors; call `reset()` afterwards.  Raises ValueError for a bad seed, an empty list, or a seed whose
+        layout routine raises or never returns in the reference (the pool is then unusable until the next upload or
+        generation)."""
+        if difficulty not in self.DIFFICULTY_IDS:
+            raise ValueError(f"Unknown difficulty: {difficulty}")
+        if isinstance(seeds, (str, bytes)):
+            raise ValueError("seeds must be an iterable of ints")
+        try:
+            seeds = [operator.index(s) for s in seeds]
+        except TypeError as e:
+            raise ValueError(f"seeds must be ints in [0, 2^64): {e}") from None
+        if not seeds:
+            raise ValueError("seeds is empty")
+        bad = next((s for s in seeds if not 0 <= s < 2**64), None)
+        if bad is not None:
+            raise ValueError(f"seed {bad} is outside [0, 2^64)")
+        arr = np.array(seeds, dtype=np.uint64)
+        try:
+            _lib.check(self._lib.merlin_env_generate_seeded_layouts(self._h, self.DIFFICULTY_IDS[difficulty],
+                                                                    arr.ctypes.data, len(seeds), self._stream()))
+        finally:
+            self.n_layouts = int(self._lib.merlin_env_layout_count(self._h))
+            self._pool_cells_host = None
 
     def layouts_numpy(self):
         """Host copy of the current pool: (cells u8[L, H*W], agent i32[L, 3])."""

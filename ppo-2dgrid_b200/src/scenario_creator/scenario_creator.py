@@ -83,8 +83,11 @@ class ScenarioCreator:
                            want_symbolic=False, n_layouts=None, **env_kwargs):
         """N envs of `difficulty` on `device`.  Layout pool: `layouts=(cells u8[L, H*W], agent i32[L, 3])`, or
         generated on the host from `seeds` (one `reset(seed=s)` layout per seed; default: seeds 0..max(N, 1024)-1).
-        `layouts="device"`: the pool (`n_layouts` entries, default max(N, 1024)) is generated on the GPU from the integer
-        `seeds` -- fresh layouts of the right distribution, not the reference's per-seed layouts.
+        `layouts="device"` generates the pool on the GPU instead:
+          - `seeds` a sequence of ints: one `reset(seed=s)` layout per seed, the same pool `layouts=None` builds on the
+            host (`n_layouts` is ignored, as there);
+          - `seeds` an int or None: `n_layouts` entries (default max(N, 1024)) from a counter-based stream keyed by the
+            int -- fresh layouts of the right distribution, not the reference's per-seed layouts.
         `fomaml_mode`: finished envs restart on their own layout (src/fomaml.py:92) instead of the next one."""
         from merlin_b200 import BatchedMerlinEnv
         from merlin_b200 import layouts as _layouts
@@ -97,7 +100,10 @@ class ScenarioCreator:
         if isinstance(layouts, str):
             if layouts != "device":
                 raise ValueError("layouts must be (cells, agent), None (host-generated from seeds) or 'device'")
-            pool = dict(generate=(diff, int(seeds or 0), int(n_layouts or max(int(num_envs), 1024))))
+            if seeds is None or np.ndim(seeds) == 0:
+                pool = dict(generate=(diff, int(seeds or 0), int(n_layouts or max(int(num_envs), 1024))))
+            else:
+                pool = dict(generate_seeded=(diff, seeds))
             cells = agent = None
         else:
             if layouts is None:
