@@ -189,6 +189,7 @@ class OracleVecEnv:
                           _p(self.carry_c), _p(actions), _p(reward), _p(term), _p(trunc))
         if r != 0:
             raise RuntimeError(f"fo_step failed: {r}")
+        reward_env = reward  # MiniGridEnv's own reward, before the shaping wrappers
         stuck = np.zeros(N, bool)
         if self.stuck_on:
             same = (self.ax == self.last_x) & (self.ay == self.last_y)
@@ -211,7 +212,7 @@ class OracleVecEnv:
             self._load(np.nonzero(done)[0])
         rgb, sym = self.observe()
         info = {"episode_return": ep_ret, "episode_length": ep_len, "stuck": stuck, "obs_symbolic": sym,
-                "reward_f64": reward}
+                "reward_f64": reward, "reward_env": reward_env}
         return rgb, reward32, term.astype(bool), trunc.astype(bool), info
 
 

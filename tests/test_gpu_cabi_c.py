@@ -14,11 +14,10 @@ pytestmark = pytest.mark.gpu
 ROOT = os.path.abspath(os.path.join(os.path.dirname(__file__), ".."))
 
 
-def test_c_program_links_and_runs_against_the_shared_library():
+def test_c_program_links_and_runs_against_the_shared_library(tmp_path):
     from merlin_b200 import _lib
     _lib.load()
-    out = os.path.join(ROOT, "tests", "csrc", "_build", "cabi_smoke")
-    os.makedirs(os.path.dirname(out), exist_ok=True)
+    out = str(tmp_path / "cabi_smoke")   # built outside the repository tree, which may be read-only
     libdir = os.path.dirname(_lib.LIB_PATH)
     subprocess.check_call(["gcc", os.path.join(ROOT, "tests", "csrc", "cabi_smoke.c"), "-I" + os.path.join(ROOT, "include"),
                            "-I/usr/local/cuda/include", "-L" + libdir, "-lmerlin_b200", "-L/usr/local/cuda/lib64", "-lcudart",

@@ -326,6 +326,85 @@ def test_sampler_frequencies_follow_softmax():
     assert ((a >= 0) & (a < 3)).all()
 
 
+def test_vectorised_uniforms_equal_the_scalar_restatement_and_known_answers():
+    """uniform_batch (uint64 numpy Philox) == the pinned scalar restatement and the header, on keys whose high word
+    matters, draw numbers past 2^31 and env indices up to 2^20; philox4x32_10_batch reproduces the Random123 vectors."""
+    from oracle import sampler
+    for ctr, key, want in PHILOX_KAT:
+        got = sampler.philox4x32_10_batch([np.full(3, c) for c in ctr], key)
+        assert all((w == np.uint64(x)).all() for w, x in zip(got, want))
+    rng = np.random.default_rng(11)
+    envs = np.concatenate([[0, 1, (1 << 20) - 1, 1 << 20], rng.integers(0, (1 << 20) + 1, 600)])
+    draws = np.concatenate([[0, (1 << 31) - 1, 1 << 31, (1 << 32) - 1], rng.integers(0, 1 << 32, 600)])
+    for seed in (0x9E3779B97F4A7C15, 0xFFFFFFFF00000000, 1 << 32, 0x1234_5678_9ABC_DEF0, 7):
+        u = sampler.uniform_batch(seed, envs, draws)
+        want = np.array([sampler.uniform(seed, int(e), int(d)) for e, d in zip(envs, draws)], np.float32)
+        assert u.dtype == np.float32 and np.array_equal(u, want), hex(seed)
+    # the header draws the same uniforms (hm_sample takes env = row index: the first 2^12 envs, draws past 2^31)
+    seed = 0x9E3779B97F4A7C15
+    d = rng.integers(1 << 31, 1 << 32, 4096)
+    _, _, u_hdr = _hm_sample(np.zeros((4096, 3), np.float32), seed, d)
+    assert np.array_equal(u_hdr, sampler.uniform_batch(seed, np.arange(4096), d))
+    # the high word of the key changes the stream
+    assert not np.array_equal(sampler.uniform_batch(seed, np.arange(64), 0),
+                              sampler.uniform_batch(seed & 0xFFFFFFFF, np.arange(64), 0))
+
+
+def _edge_rows(A):
+    """Finite edge rows (ties, spreads from 100 to 6e38 = 3e38 - -3e38, -inf logits) with `A` actions."""
+    rows = [[1.0] * A, [2.0] + [5.0] * (A - 1), [5.0] * (A - 1) + [2.0], [0.0] * (A - 1) + [3.0]]
+    for s in (100.0, 1e3, 1e5, 1e10, 1e20, 3e38):
+        rows += [[s] + [0.0] * (A - 2) + [-s], [-s] + [0.0] * (A - 2) + [s], [0.0] * (A - 1) + [-s],
+                 [0.0, -s] + [0.0] * (A - 2)]
+    ninf = -np.inf
+    rows += [[ninf] + [0.0] * (A - 1), [0.0, ninf] + [1.0] * (A - 2), [1.0] * (A - 1) + [ninf],
+             [ninf] * (A - 1) + [0.5], [2.0, ninf] + [2.0] * (A - 2), [ninf, 1e30] + [-1e30] * (A - 2)]
+    return np.asarray(rows, np.float32)
+
+
+@pytest.mark.parametrize("A", [3, 7])
+def test_sampler_header_obeys_the_float64_reference_on_edge_rows(A):
+    """sample_policy (host build of the header) on edge rows, every row drawn with 2000 draw numbers: the action is one
+    reference_f64 allows for the header's own uniform (a -inf logit is never drawn), the log-probability is finite and
+    within float32 rounding of log_softmax in float64, and greedy picks the first maximum."""
+    from oracle import sampler
+    rows = _edge_rows(A)
+    R, D = len(rows), 2000
+    logits = np.repeat(rows, D, axis=0)
+    draws = np.tile(np.arange(D), R) * 7919
+    act, lp, u = _hm_sample(logits, 0x9E3779B97F4A7C15, draws)
+    _, logp64, allowed = sampler.reference_f64(logits, u)
+    n = np.arange(len(logits))
+    assert allowed[n, act].all(), np.unique(np.nonzero(~allowed[n, act])[0] // D)
+    assert not np.isneginf(logits[n, act]).any()
+    assert np.isfinite(lp).all()
+    l64 = logits.astype(np.float64)
+    z = l64[n, act] - l64.max(axis=1)
+    lse = np.log(np.exp(l64 - l64.max(axis=1, keepdims=True)).sum(axis=1))
+    assert (np.abs(lp - logp64[n, act]) <= 2e-6 + 4 * 2.0 ** -24 * (np.abs(z) + np.abs(lse))).all()
+    g_act, g_lp, _ = _hm_sample(rows, 1, np.zeros(R), greedy=True)
+    assert np.array_equal(g_act, np.argmax(rows, axis=1))   # first maximum, ties included
+    assert np.isfinite(g_lp).all()
+
+
+@pytest.mark.parametrize("A", [3, 7])
+def test_sampler_header_non_finite_rows_stay_in_range(A):
+    """NaN, +inf and all -inf rows: what is specified is an action in [0, A).  The header falls back to the last action
+    with logp = NaN when sampling; greedy skips a NaN after the first logit, and a NaN first logit wins."""
+    nan, inf = np.nan, np.inf
+    rows = np.asarray([[nan] + [0.0] * (A - 1), [0.0, nan] + [1.0] * (A - 2), [0.0] * (A - 1) + [nan],
+                       [0.0, inf] + [0.0] * (A - 2), [inf] * A, [-inf] * A, [inf, -inf] + [nan] * (A - 2),
+                       [-inf] * (A - 1) + [inf]], np.float32)
+    R = len(rows)
+    logits = np.repeat(rows, 500, axis=0)
+    act, lp, _ = _hm_sample(logits, 0x9E3779B97F4A7C15, np.arange(len(logits)))
+    assert ((act >= 0) & (act < A)).all()
+    assert (act == A - 1).all() and np.isnan(lp).all()
+    g_act, _, _ = _hm_sample(rows, 0, np.zeros(R), greedy=True)
+    assert ((g_act >= 0) & (g_act < A)).all()
+    assert g_act[0] == 0 and g_act[1] == 2 and g_act[3] == 1 and g_act[4] == 0 and g_act[7] == A - 1
+
+
 # ---- property tests (hypothesis): arbitrary W x H rooms, full object set, arbitrary action strings ----------------
 from hypothesis import HealthCheck, given, settings, strategies as st  # noqa: E402
 
