@@ -18,6 +18,8 @@
  *   merlin_env_step               env.step(a)   src/ppo.py:76 ; src/fomaml.py:71 -- through
  *                                 ThreeActionWrapper (src/wrappers/three_action_wrapper.py:10-17),
  *                                 optionally StuckPenaltyWrapper (src/wrappers/stuck_penalty_wrapper.py:29-58)
+ *   merlin_env_step_final / merlin_env_policy_step_final   the same two, also returning the observation of every
+ *                                 terminal state before its auto-reset (src/ppo.py:76,93-96: env.step(a), then env.reset())
  *   merlin_env_policy_step        the whole rollout transition "act -> sample -> step -> store": Categorical(logits).sample(),
  *                                 .log_prob(a) (src/actor_critic.py:80-99 act()), env.step(a) and RolloutBuffer.add /
  *                                 the trajectory lists (src/ppo.py:70-86 ; src/fomaml.py:65-84) in ONE launch; with
@@ -196,6 +198,22 @@ int merlin_env_policy_step(merlin_env_t* h, const merlin_policy_io_t* policy, ui
                            float* reward, uint8_t* terminated, uint8_t* truncated, const merlin_step_extras_t* extras,
                            void* stream);
 int merlin_env_seed_sampler(merlin_env_t* h, uint64_t seed);
+
+/* Final observations of auto-reset episodes (gymnasium's info["final_obs"]; what the reference's env.step(a) returns
+ * before its caller runs env.reset(), src/ppo.py:76,93-96).  merlin_env_step / merlin_env_policy_step plus
+ *   final_sym   DEVICE u8[N][7][7][3]: when env e's episode ends in this step (terminated or truncated), row e receives
+ *               the Grid.encode image of env e's state after the action and before the auto-reset -- byte for byte the
+ *               obs_sym row the same step writes with MERLIN_F_AUTO_RESET off.  Rows of the other envs are not written.
+ * Every other output, the env state and the draw counters are exactly those of the call without final_sym;
+ * final_sym == NULL is that call.  Asynchronous, allocates nothing, capturable.  No RGB frame is written for the
+ * terminal state: merlin_env_render(final_sym, index = the done rows) gives exactly the frame such a step would write.
+ * Time-limit bootstrapping (reward += gamma * V(final observation) on truncated steps) needs this image. */
+int merlin_env_step_final(merlin_env_t* h, const int64_t* actions, uint8_t* obs_rgb, uint8_t* obs_sym, float* reward,
+                          uint8_t* terminated, uint8_t* truncated, const merlin_step_extras_t* extras,
+                          uint8_t* final_sym, void* stream);
+int merlin_env_policy_step_final(merlin_env_t* h, const merlin_policy_io_t* policy, uint8_t* obs_rgb,
+                                 uint8_t* obs_sym, float* reward, uint8_t* terminated, uint8_t* truncated,
+                                 const merlin_step_extras_t* extras, uint8_t* final_sym, void* stream);
 /* Clear the in-kernel work-ticket counters of this handle on `stream` (see Conventions). */
 int merlin_env_rearm(merlin_env_t* h, void* stream);
 
@@ -257,6 +275,9 @@ int merlin_set_kernel_choice(int choice);
 int merlin_set_observation_path(int path);
 /* Name of the kernel merlin_env_step launches for this handle (rgb != 0: with an RGB observation). */
 const char* merlin_env_step_kernel(merlin_env_t* h, int rgb);
+/* The same for merlin_env_step_final / merlin_env_policy_step_final with a final_sym buffer (kernel choice 7 runs the
+ * warp-per-env kernel there). */
+const char* merlin_env_final_step_kernel(merlin_env_t* h, int rgb);
 
 /* GAE + returns over a time-major [T][N] rollout (all DEVICE f32). done = terminated|truncated as 0/1.
  * adv[t] = delta_t + gamma*lam*(1-done_t)*adv[t+1]; ret = val + adv.  fp32, unfused, reference op order.

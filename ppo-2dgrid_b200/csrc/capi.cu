@@ -494,7 +494,7 @@ int merlin_env_reset(merlin_env_t* h, const uint8_t* mask, uint8_t* obs_rgb, uin
 
 static int step_common(merlin_env_t* h, const int64_t* actions, const merlin_policy_io_t* pol, uint8_t* obs_rgb,
                        uint8_t* obs_sym, float* reward, uint8_t* terminated, uint8_t* truncated,
-                       const merlin_step_extras_t* extras, void* stream) {
+                       const merlin_step_extras_t* extras, uint8_t* final_sym, void* stream) {
   if (!reward || !terminated || !truncated) return fail(MERLIN_EINVAL, "reward/terminated/truncated are required");
   if (!h->was_reset) return fail(MERLIN_ESTATE, "step before reset");
   if (obs_rgb && !h->has_atlas) return fail(MERLIN_ESTATE, "RGB observation requested before the tile atlas was set");
@@ -503,6 +503,7 @@ static int step_common(merlin_env_t* h, const int64_t* actions, const merlin_pol
   EnvParams p = base_params(h);
   p.actions = actions; p.obs_rgb = obs_rgb; p.obs_sym = obs_sym;
   p.reward = reward; p.terminated = terminated; p.truncated = truncated;
+  p.final_sym = final_sym;
   if (extras) { p.out_ep_return = extras->episode_return; p.out_ep_length = extras->episode_length; p.out_stuck = extras->stuck; p.out_done = extras->done; }
   if (pol) {
     p.logits = pol->logits; p.value_in = pol->value; p.out_action = pol->action; p.out_logp = pol->logprob;
@@ -524,13 +525,18 @@ int merlin_env_step(merlin_env_t* h, const int64_t* actions, uint8_t* obs_rgb, u
                     uint8_t* terminated, uint8_t* truncated, const merlin_step_extras_t* extras, void* stream) {
   if (!h) return fail(MERLIN_EINVAL, "null handle");
   if (!actions) return fail(MERLIN_EINVAL, "actions/reward/terminated/truncated are required");
-  return step_common(h, actions, nullptr, obs_rgb, obs_sym, reward, terminated, truncated, extras, stream);
+  return step_common(h, actions, nullptr, obs_rgb, obs_sym, reward, terminated, truncated, extras, nullptr, stream);
 }
 
-int merlin_env_policy_step(merlin_env_t* h, const merlin_policy_io_t* pol, uint8_t* obs_rgb, uint8_t* obs_sym,
-                           float* reward, uint8_t* terminated, uint8_t* truncated, const merlin_step_extras_t* extras,
-                           void* stream) {
+int merlin_env_step_final(merlin_env_t* h, const int64_t* actions, uint8_t* obs_rgb, uint8_t* obs_sym, float* reward,
+                          uint8_t* terminated, uint8_t* truncated, const merlin_step_extras_t* extras,
+                          uint8_t* final_sym, void* stream) {
   if (!h) return fail(MERLIN_EINVAL, "null handle");
+  if (!actions) return fail(MERLIN_EINVAL, "actions/reward/terminated/truncated are required");
+  return step_common(h, actions, nullptr, obs_rgb, obs_sym, reward, terminated, truncated, extras, final_sym, stream);
+}
+
+static int check_policy_io(merlin_env_t* h, const merlin_policy_io_t* pol) {
   if (!pol || !pol->logits || !pol->action || !pol->logprob)
     return fail(MERLIN_EINVAL, "merlin_env_policy_step: logits, action and logprob are required");
   if (pol->value_out && !pol->value) return fail(MERLIN_EINVAL, "merlin_env_policy_step: value_out needs value");
@@ -539,7 +545,23 @@ int merlin_env_policy_step(merlin_env_t* h, const merlin_policy_io_t* pol, uint8
     return fail(MERLIN_EINVAL, "merlin_env_policy_step: logits_stride smaller than the action count");
   if (pol->finished && (!pol->first_return || !pol->first_length || !pol->first_goal))
     return fail(MERLIN_EINVAL, "merlin_env_policy_step: the first-episode record needs all four arrays");
-  return step_common(h, nullptr, pol, obs_rgb, obs_sym, reward, terminated, truncated, extras, stream);
+  return MERLIN_OK;
+}
+
+int merlin_env_policy_step(merlin_env_t* h, const merlin_policy_io_t* pol, uint8_t* obs_rgb, uint8_t* obs_sym,
+                           float* reward, uint8_t* terminated, uint8_t* truncated, const merlin_step_extras_t* extras,
+                           void* stream) {
+  if (!h) return fail(MERLIN_EINVAL, "null handle");
+  if (const int rc = check_policy_io(h, pol)) return rc;
+  return step_common(h, nullptr, pol, obs_rgb, obs_sym, reward, terminated, truncated, extras, nullptr, stream);
+}
+
+int merlin_env_policy_step_final(merlin_env_t* h, const merlin_policy_io_t* pol, uint8_t* obs_rgb, uint8_t* obs_sym,
+                                 float* reward, uint8_t* terminated, uint8_t* truncated,
+                                 const merlin_step_extras_t* extras, uint8_t* final_sym, void* stream) {
+  if (!h) return fail(MERLIN_EINVAL, "null handle");
+  if (const int rc = check_policy_io(h, pol)) return rc;
+  return step_common(h, nullptr, pol, obs_rgb, obs_sym, reward, terminated, truncated, extras, final_sym, stream);
 }
 
 int merlin_env_seed_sampler(merlin_env_t* h, uint64_t seed) {
@@ -685,7 +707,14 @@ int64_t merlin_env_launch_count(merlin_env_t* h) { return h ? h->launches : 0; }
 
 const char* merlin_env_step_kernel(merlin_env_t* h, int rgb) {
   if (!h) return "";
-  return step_kernel_name(select_step_kernel(h->cfg.n_envs, (rgb & 1) != 0, lean_config(h->cfg.flags), launch_ctx(h)));
+  return step_kernel_name(
+      select_step_kernel(h->cfg.n_envs, (rgb & 1) != 0, lean_config(h->cfg.flags), false, launch_ctx(h)));
+}
+
+const char* merlin_env_final_step_kernel(merlin_env_t* h, int rgb) {
+  if (!h) return "";
+  return step_kernel_name(
+      select_step_kernel(h->cfg.n_envs, (rgb & 1) != 0, lean_config(h->cfg.flags), true, launch_ctx(h)));
 }
 
 static int check_kernel_choice(int choice, int lowest) {

@@ -5,9 +5,10 @@
 // helpers in env_kernels_common.cuh, the lane-per-env state phase in env_state_phase.cuh.
 //
 // Every step kernel does the same work per environment -- step + wrappers + auto-reset (STEP = 1: actions given;
-// STEP = 2: actions drawn in the kernel from the policy's logits, merlin_env_policy_step) or a masked reset (STEP = 0),
-// then gen_obs (+process_vis), the symbolic encode and the RGB frame -- and differs only in how environments are mapped
-// onto the machine.  Two phases:
+// STEP = 2: actions drawn in the kernel from the policy's logits, merlin_env_policy_step; STEP = 3 / 4: the same two,
+// also writing the symbolic image of every terminal state before its restart) or a masked reset (STEP = 0), then
+// gen_obs (+process_vis), the symbolic encode and the RGB frame -- and differs only in how environments are mapped onto
+// the machine.  Two phases:
 //
 //   state phase   step logic, reward shaping, restart, 49-cell window gather, bitmask visibility -> the 49 tile
 //                 kinds (and 147 symbolic bytes) of the env, in shared memory.  ~20 warp-instructions per env when
@@ -220,7 +221,7 @@ static cudaError_t launch_ordered_kernel(const EnvParams& p, const LaunchCtx& ct
 constexpr int kRgbWarpMaxEnvs = 24576;
 constexpr int kSymWarpMaxEnvs = 2048;
 
-StepKernel select_step_kernel(int n_envs, bool rgb, bool lean, const LaunchCtx& ctx) {
+StepKernel select_step_kernel(int n_envs, bool rgb, bool lean, bool final, const LaunchCtx& ctx) {
   int choice = ctx.kernel_choice;
   if (choice == kChoiceAuto) {
     if (rgb) choice = n_envs <= kRgbWarpMaxEnvs ? kChoiceWarp : kChoiceTile;
@@ -238,7 +239,7 @@ StepKernel select_step_kernel(int n_envs, bool rgb, bool lean, const LaunchCtx& 
       // tiles of 16 envs once every resident CTA gets one; smaller tiles spread a small batch over more CTAs
       return {kChoiceTile, n_envs >= ctx.sm_count * kTileCtasPerSm * 16 ? 16 : 8};
     case kChoiceQuad:
-      return {lean && rgb ? kChoiceQuad : kChoiceWarp, 0};
+      return {lean && rgb && !final ? kChoiceQuad : kChoiceWarp, 0};
     default:
       return {choice, 0};
   }
@@ -260,7 +261,7 @@ const char* step_kernel_name(StepKernel k) {
 
 template <int STEP>
 static cudaError_t launch_sized(const EnvParams& p, const LaunchCtx& ctx, cudaStream_t stream) {
-  const StepKernel k = select_step_kernel(p.N, p.obs_rgb != nullptr, lean_config(p.flags), ctx);
+  const StepKernel k = select_step_kernel(p.N, p.obs_rgb != nullptr, lean_config(p.flags), step_final(STEP), ctx);
   switch (k.choice) {
     case kChoiceGroup:
       if (k.size == 32) return launch_group_kernel<32, STEP>(p, ctx, stream);
@@ -272,13 +273,14 @@ static cudaError_t launch_sized(const EnvParams& p, const LaunchCtx& ctx, cudaSt
     case kChoiceSym: return launch_sym_kernel<STEP>(p, ctx, stream);
     case kChoiceOrdered: return launch_ordered_kernel<STEP>(p, ctx, stream);
     case kChoiceQuad:
-      if (STEP != 0) return launch_quad_kernel(STEP, p, ctx, stream);
-      return launch_warp_kernel(STEP, p, ctx, stream);   // the quad kernel only steps
+      if (STEP == 1 || STEP == 2) return launch_quad_kernel(STEP, p, ctx, stream);
+      return launch_warp_kernel(STEP, p, ctx, stream);   // the quad kernel only steps, without final observations
     default: return launch_warp_kernel(STEP, p, ctx, stream);
   }
 }
 
 cudaError_t launch_env_step(const EnvParams& p, const LaunchCtx& ctx, cudaStream_t stream) {
+  if (p.final_sym != nullptr) return p.logits != nullptr ? launch_sized<4>(p, ctx, stream) : launch_sized<3>(p, ctx, stream);
   return p.logits != nullptr ? launch_sized<2>(p, ctx, stream) : launch_sized<1>(p, ctx, stream);
 }
 cudaError_t launch_env_reset(const EnvParams& p, const LaunchCtx& ctx, cudaStream_t stream) {

@@ -66,6 +66,10 @@ struct EnvParams {
   float* rec_return;           // [N]
   int32_t* rec_length;         // [N]
   uint8_t* rec_goal;           // [N] 1 = the episode ended by termination with a positive reward (goal reached)
+  // final observations (STEP = 3 / 4 instances only): when env e's episode ends in this step, row e receives the
+  // Grid.encode image of its state after the action and before the auto-reset; other rows are not written.  Kept last:
+  // a field inserted earlier would move every parameter offset of the existing instances.
+  uint8_t* final_sym;          // [N][147]
 };
 
 // Resident CTAs per SM of every kernel instance a handle has launched eagerly, keyed by the kernel's address (graph
@@ -109,12 +113,13 @@ inline bool lean_config(uint32_t flags) {
 }
 
 // The step kernel a step of n_envs envs runs: `choice` is never kChoiceAuto, `size` is G (kChoiceGroup) or T
-// (kChoiceTile) and 0 otherwise.  A reset sent to kChoiceQuad runs kChoiceWarp.
+// (kChoiceTile) and 0 otherwise.  A reset, or a step that records final observations (`final`), sent to kChoiceQuad
+// runs kChoiceWarp.
 struct StepKernel {
   int choice;
   int size;
 };
-StepKernel select_step_kernel(int n_envs, bool rgb, bool lean, const LaunchCtx& ctx);
+StepKernel select_step_kernel(int n_envs, bool rgb, bool lean, bool final, const LaunchCtx& ctx);
 const char* step_kernel_name(StepKernel k);
 cudaError_t launch_env_step(const EnvParams& p, const LaunchCtx& ctx, cudaStream_t stream);
 cudaError_t launch_env_reset(const EnvParams& p, const LaunchCtx& ctx, cudaStream_t stream);

@@ -73,11 +73,15 @@ struct ActionDraw {
   float logp;
   uint32_t draw;
 };
-// The step kernels are instantiated three times: STEP = 0 (masked reset), 1 (step, actions given), 2 (step, actions
-// drawn here from the policy's logits).  The policy code exists only in the STEP = 2 instances: compiled into the
-// others -- even behind a uniform branch, even out of line -- it degrades the register allocation of the frame kernels'
-// state phase, which runs under a 128-register cap (B200, 1M envs: 1461 us per step vs 1434 us without it;
-// profiles/r02_tile_kernel_ab.txt).
+// The step kernels are instantiated five times: STEP = 0 (masked reset), 1 (step, actions given), 2 (step, actions
+// drawn here from the policy's logits), 3 and 4 (1 and 2 that also write the final observation of every episode that
+// ends, EnvParams::final_sym).  The policy code exists only in the instances that draw, the final-observation code only
+// in STEP 3 / 4: compiled into the others -- even behind a uniform branch, even out of line -- it degrades the register
+// allocation of the frame kernels' state phase, which runs under a 128-register cap (B200, 1M envs: 1461 us per step vs
+// 1434 us without the policy code; profiles/r02_tile_kernel_ab.txt).
+__host__ __device__ constexpr bool step_given(int STEP) { return STEP == 1 || STEP == 3; }   // actions from `actions`
+__host__ __device__ constexpr bool step_draws(int STEP) { return STEP == 2 || STEP == 4; }   // drawn from `logits`
+__host__ __device__ constexpr bool step_final(int STEP) { return STEP >= 3; }                // writes `final_sym`
 template <bool POLICY>
 __device__ __forceinline__ ActionDraw draw_action(const EnvParams& p, int n_actions, int e) {
   ActionDraw d;
@@ -199,7 +203,8 @@ static cudaError_t resident_ctas(const LaunchCtx& ctx, Kernel kernel, int thread
   return cudaSuccess;
 }
 
-// small-batch step kernels (env_kernels_small.cu); `step` = 0 masked reset, 1 step with given actions, 2 policy step
+// small-batch step kernels (env_kernels_small.cu); `step` = 0 masked reset, 1 step with given actions, 2 policy step,
+// 3 / 4 the same two recording final observations
 cudaError_t launch_warp_kernel(int step, const EnvParams& p, const LaunchCtx& ctx, cudaStream_t stream);
 cudaError_t launch_quad_kernel(int step, const EnvParams& p, const LaunchCtx& ctx, cudaStream_t stream);   // step 1 or 2
 

@@ -35,6 +35,28 @@ constexpr int kWarpPdlMinEnvs = 4096;
 constexpr int kWarpKindBytes = 128;          // 49 premultiplied kinds (u16) per warp, padded
 constexpr int kPairChunks = 2 * kUnitsPerRow / 2;   // 21 16-byte chunks per pair of pixel rows
 
+// Final observation of one env, one warp per env (STEP = 3 / 4): the 49 window codes of its terminal state, code0 in
+// mask order c = lane and code1 at c = lane + 32, encoded into the global row `out` -- the same ballots, visibility and
+// bytes as the observation part of env_kernel_warp.
+__device__ __forceinline__ void warp_store_final(uint32_t code0, uint32_t code1, int lane, uint32_t carry, uint8_t* out) {
+  const int c1 = lane + 32;
+  const unsigned t0 = __ballot_sync(0xffffffffu, !((M_OPAQUE >> (code0 & 0xf)) & 1u));
+  const unsigned t1 = __ballot_sync(0xffffffffu, c1 < kCells && !((M_OPAQUE >> (code1 & 0xf)) & 1u));
+  const uint64_t vis = visibility((uint64_t)t0 | ((uint64_t)t1 << 32));
+#pragma unroll
+  for (int h = 0; h < 2; ++h) {
+    const int c = h ? c1 : lane;
+    if (c >= kCells) break;
+    const int vj = (c * 37) >> 8, vi = c - vj * kView;   // c / 7 for c < 64
+    const bool agent_cell = (vi == kView / 2 && vj == kView - 1);
+    const uint32_t code = agent_cell ? (carry ? carry : CODE_EMPTY) : (h ? code1 : code0);
+    uint8_t t = 0, col = 0, stt = 0;
+    if ((vis >> c) & 1) sym_of_code(code, t, col, stt);
+    uint8_t* o = out + (vi * kView + vj) * 3;
+    o[0] = t; o[1] = col; o[2] = stt;
+  }
+}
+
 template <int STEP, bool PDL, bool LEAN = false>
 __global__ void __launch_bounds__(kWarpKernelThreads, kWarpCtas) env_kernel_warp(const EnvParams p) {
   extern __shared__ __align__(16) uint8_t smem[];
@@ -63,7 +85,7 @@ __global__ void __launch_bounds__(kWarpKernelThreads, kWarpCtas) env_kernel_warp
   } else if (e < p.N) {
     // first env's state / action: in flight while the atlas is staged
     st_next = p.state[e];
-    if (STEP == 1) act_next = p.actions[e];
+    if (step_given(STEP)) act_next = p.actions[e];
   }
   if (f.want_rgb) {
     // thread t tests tile t / 2 and copies half of it (6 int4); a 128-thread CTA takes two rounds
@@ -81,7 +103,7 @@ __global__ void __launch_bounds__(kWarpKernelThreads, kWarpCtas) env_kernel_warp
     asm volatile("griddepcontrol.wait;" ::: "memory");
     if (e < p.N) {
       st_next = p.state[e];
-      if (STEP == 1) act_next = p.actions[e];
+      if (step_given(STEP)) act_next = p.actions[e];
     }
   }
   __syncthreads();
@@ -111,7 +133,7 @@ __global__ void __launch_bounds__(kWarpKernelThreads, kWarpCtas) env_kernel_warp
       const int en = e + gridDim.x * warps_per_cta;   // prefetch the next env of this warp
       if (en < p.N) {
         st_next = p.state[en];
-        if (STEP == 1) act_next = p.actions[en];
+        if (step_given(STEP)) act_next = p.actions[en];
       }
     }
     unpack_state(st.x, st.y, st.z, st.w, s);
@@ -128,7 +150,7 @@ __global__ void __launch_bounds__(kWarpKernelThreads, kWarpCtas) env_kernel_warp
       // of an agent that moved is ext rows 0..6 (cell c = x: the lane's own loads); of one that did not, rows 1..7
       // (c = x - 7: one lane rotation by 7).
       ActionDraw act;
-      if (STEP == 2) act = draw_action<true>(p, 3, e);
+      if (step_draws(STEP)) act = draw_action<true>(p, 3, e);
       else { act.action = act_in; act.logp = 0.f; act.draw = 0; }
       const bool bad = act.action < 0 || act.action >= 3;
       const int a = bad ? A_DONE : (int)act.action;
@@ -157,8 +179,8 @@ __global__ void __launch_bounds__(kWarpKernelThreads, kWarpCtas) env_kernel_warp
       ep_ret += rew;
       const bool done = terminated || truncated;
       if (lane == 0) {
-        commit_action<STEP == 2>(p, e, act);
-        record_first_episode<STEP == 2>(p, e, done, goal && rew > 0.f, ep_ret, s.step_count);
+        commit_action<step_draws(STEP)>(p, e, act);
+        record_first_episode<step_draws(STEP)>(p, e, done, goal && rew > 0.f, ep_ret, s.step_count);
         if (bad) atomicAdd(p.bad_actions, 1ull);
         p.reward[e] = rew;
         p.terminated[e] = terminated ? 1 : 0;
@@ -173,6 +195,10 @@ __global__ void __launch_bounds__(kWarpKernelThreads, kWarpCtas) env_kernel_warp
       const uint32_t r0 = __shfl_sync(0xffffffffu, e0, rot), r1 = __shfl_sync(0xffffffffu, e1, rot);
       code0 = moved ? e0 : (lane + kView < 32 ? r0 : r1);
       code1 = moved ? e1 : r1;
+      // the window just assembled is the terminal state's: its final image, before the restart below (warp-uniform)
+      if constexpr (step_final(STEP)) {
+        if (done) warp_store_final(code0, code1, lane, s.carry, p.final_sym + (size_t)e * kSymBytes);
+      }
     } else if (STEP) {
       const uint8_t* grid = f.mutable_grid ? p.cells + (size_t)e * p.cell_stride
                                            : p.pool_cells + (size_t)s.layout * p.cell_stride;
@@ -181,7 +207,7 @@ __global__ void __launch_bounds__(kWarpKernelThreads, kWarpCtas) env_kernel_warp
       const int fidx = fy * p.W + fx;
       const uint32_t fwd = inb ? ld_cell(grid + fidx, f.pol) : CODE_WALL;
       ActionDraw act;
-      if (STEP == 2) act = draw_action<true>(p, f.n_actions, e);
+      if (step_draws(STEP)) act = draw_action<true>(p, f.n_actions, e);
       else { act.action = act_in; act.logp = 0.f; act.draw = 0; }
       StepResult r = step_logic(s, act.action, f.n_actions, fwd, inb, fidx, p.max_steps);
       uint32_t vword = 0;
@@ -197,8 +223,8 @@ __global__ void __launch_bounds__(kWarpKernelThreads, kWarpCtas) env_kernel_warp
       const bool done = r.terminated || r.truncated;
       __syncwarp();  // every lane has read the old grid cell / visited word / draw counter before lane 0 overwrites them
       if (lane == 0) {
-        commit_action<STEP == 2>(p, e, act);
-        record_first_episode<STEP == 2>(p, e, done, r.terminated && r.reward > 0.0, ep_ret, s.step_count);
+        commit_action<step_draws(STEP)>(p, e, act);
+        record_first_episode<step_draws(STEP)>(p, e, done, r.terminated && r.reward > 0.0, ep_ret, s.step_count);
         if (r.bad_action) atomicAdd(p.bad_actions, 1ull);
         if (r.write_idx >= 0 && f.mutable_grid) p.cells[(size_t)e * p.cell_stride + r.write_idx] = (uint8_t)r.write_code;
         if (f.explore_on && vword != vword_in) *vptr = vword;
@@ -209,6 +235,23 @@ __global__ void __launch_bounds__(kWarpKernelThreads, kWarpCtas) env_kernel_warp
         if (p.out_ep_length) p.out_ep_length[e] = done ? s.step_count : 0;
         if (p.out_stuck) p.out_stuck[e] = stuck ? 1 : 0;
         if (p.out_done) p.out_done[e] = done ? 1.f : 0.f;
+      }
+      // final image (warp-uniform): the window after lane 0's grid write above, before the restart copy below
+      if constexpr (step_final(STEP)) {
+        if (done) {
+          __syncwarp();
+          const int fx = dir_dx(s.dir), fy = dir_dy(s.dir);
+          uint32_t w0, w1 = CODE_WALL;
+          {
+            const int wx = s.x + a0 * fx - b0 * fy, wy = s.y + a0 * fy + b0 * fx;
+            w0 = ((unsigned)wx < (unsigned)p.W && (unsigned)wy < (unsigned)p.H) ? ld_cell(grid + wy * p.W + wx, f.pol) : CODE_WALL;
+          }
+          if (c1 < kCells) {
+            const int wx = s.x + a1 * fx - b1 * fy, wy = s.y + a1 * fy + b1 * fx;
+            w1 = ((unsigned)wx < (unsigned)p.W && (unsigned)wy < (unsigned)p.H) ? ld_cell(grid + wy * p.W + wx, f.pol) : CODE_WALL;
+          }
+          warp_store_final(w0, w1, lane, s.carry, p.final_sym + (size_t)e * kSymBytes);
+        }
       }
       restart = done && f.auto_reset;
     } else {
@@ -348,7 +391,7 @@ __device__ __forceinline__ void load_ext_row(const EnvParams& p, const uint8_t* 
 
 template <int STEP, bool PDL>
 __global__ void __launch_bounds__(kWarpKernelThreads, kQuadCtas) env_kernel_quad(const EnvParams p) {
-  static_assert(STEP == 1 || STEP == 2, "the quad kernel steps; resets run the warp kernel");
+  static_assert(STEP == 1 || STEP == 2, "the quad kernel steps; resets and final-observation steps run the warp kernel");
   extern __shared__ __align__(16) uint8_t smem[];
   const int lane = threadIdx.x & 31;
   const int warp = threadIdx.x >> 5;
@@ -370,7 +413,7 @@ __global__ void __launch_bounds__(kWarpKernelThreads, kQuadCtas) env_kernel_quad
   } else if (q < n_quads) {
     const int e = min(4 * q + g, p.N - 1);
     st_next = p.state[e];
-    if (STEP == 1) act_next = p.actions[e];
+    if (step_given(STEP)) act_next = p.actions[e];
   }
   for (int t = threadIdx.x; t < 2 * kAtlasTiles; t += blockDim.x) {
     const int tile = t >> 1, half = t & 1;
@@ -386,7 +429,7 @@ __global__ void __launch_bounds__(kWarpKernelThreads, kQuadCtas) env_kernel_quad
     if (q < n_quads) {
       const int e = min(4 * q + g, p.N - 1);
       st_next = p.state[e];
-      if (STEP == 1) act_next = p.actions[e];
+      if (step_given(STEP)) act_next = p.actions[e];
     }
   }
   __syncthreads();
@@ -408,7 +451,7 @@ __global__ void __launch_bounds__(kWarpKernelThreads, kQuadCtas) env_kernel_quad
     if (q + stride < n_quads) {
       const int en = min(4 * (q + stride) + g, p.N - 1);
       st_next = p.state[en];
-      if (STEP == 1) act_next = p.actions[en];
+      if (step_given(STEP)) act_next = p.actions[en];
     }
     int x = st.x & 0xff, y = (st.x >> 8) & 0xff, dir = (st.x >> 16) & 3;
     uint32_t carry = ((uint32_t)st.x >> 24) & 0x7f;
@@ -416,7 +459,7 @@ __global__ void __launch_bounds__(kWarpKernelThreads, kQuadCtas) env_kernel_quad
     float ep_ret = p.ep_return[e];
 
     ActionDraw act;
-    if (STEP == 2) act = draw_action<true>(p, 3, e);
+    if (step_draws(STEP)) act = draw_action<true>(p, 3, e);
     else { act.action = act_in; act.logp = 0.f; act.draw = 0; }
     const bool bad = act.action < 0 || act.action >= 3;
     const int a = bad ? A_DONE : (int)act.action;
@@ -439,8 +482,8 @@ __global__ void __launch_bounds__(kWarpKernelThreads, kQuadCtas) env_kernel_quad
     ep_ret += rew;
     const bool done = terminated || truncated;
     if (r == 0 && valid) {
-      commit_action<STEP == 2>(p, e, act);
-      record_first_episode<STEP == 2>(p, e, done, goal && rew > 0.f, ep_ret, step_count);
+      commit_action<step_draws(STEP)>(p, e, act);
+      record_first_episode<step_draws(STEP)>(p, e, done, goal && rew > 0.f, ep_ret, step_count);
       if (bad) atomicAdd(p.bad_actions, 1ull);
       p.reward[e] = rew;
       p.terminated[e] = terminated ? 1 : 0;
@@ -595,6 +638,8 @@ static cudaError_t launch_quad_kernel_step(const EnvParams& p, const LaunchCtx& 
 cudaError_t launch_warp_kernel(int step, const EnvParams& p, const LaunchCtx& ctx, cudaStream_t stream) {
   if (step == 0) return launch_warp_kernel_step<0>(p, ctx, stream);
   if (step == 1) return launch_warp_kernel_step<1>(p, ctx, stream);
+  if (step == 3) return launch_warp_kernel_step<3>(p, ctx, stream);
+  if (step == 4) return launch_warp_kernel_step<4>(p, ctx, stream);
   return launch_warp_kernel_step<2>(p, ctx, stream);
 }
 cudaError_t launch_quad_kernel(int step, const EnvParams& p, const LaunchCtx& ctx, cudaStream_t stream) {

@@ -221,15 +221,21 @@ cudaError_t launch_tile_kernel(int T, int step, const EnvParams& p, const Launch
   if (T == 16) {
     if (step == 0) return launch_tile_kernel_step<16, 0>(p, ctx, stream);
     if (step == 1) return launch_tile_kernel_step<16, 1>(p, ctx, stream);
+    if (step == 3) return launch_tile_kernel_step<16, 3>(p, ctx, stream);
+    if (step == 4) return launch_tile_kernel_step<16, 4>(p, ctx, stream);
     return launch_tile_kernel_step<16, 2>(p, ctx, stream);
   }
   if (step == 0) return launch_tile_kernel_step<8, 0>(p, ctx, stream);
   if (step == 1) return launch_tile_kernel_step<8, 1>(p, ctx, stream);
+  if (step == 3) return launch_tile_kernel_step<8, 3>(p, ctx, stream);
+  if (step == 4) return launch_tile_kernel_step<8, 4>(p, ctx, stream);
   return launch_tile_kernel_step<8, 2>(p, ctx, stream);
 }
 cudaError_t launch_tile_tma_kernel(int step, const EnvParams& p, const LaunchCtx& ctx, cudaStream_t stream) {
   if (step == 0) return launch_tile_tma_kernel_step<0>(p, ctx, stream);
   if (step == 1) return launch_tile_tma_kernel_step<1>(p, ctx, stream);
+  if (step == 3) return launch_tile_tma_kernel_step<3>(p, ctx, stream);
+  if (step == 4) return launch_tile_tma_kernel_step<4>(p, ctx, stream);
   return launch_tile_tma_kernel_step<2>(p, ctx, stream);
 }
 

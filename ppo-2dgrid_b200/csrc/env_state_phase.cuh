@@ -49,6 +49,42 @@ __device__ __forceinline__ void store_sym_row(uint8_t* row, const uint64_t (&g)[
   }
 }
 
+// Grid.encode image of one env's view, cell by cell, straight into a global row: the final observation of an episode
+// that ends (STEP = 3 / 4).  Two passes over the window -- the transparency mask by view rows, then the encode by view
+// columns -- with the seven loads of a row or column in flight together: 14 round trips, and few enough registers that
+// the caller's allocation does not grow (every cell at once costs the register-capped tile and symbolic kernels
+// hundreds of bytes of spills).  Same bytes as the observation part of state_phase (either form).  About
+// N / max_steps lanes of a step take this path.
+static __device__ __noinline__ void store_final_row(const EnvState& s, const uint8_t* grid, int W, int H, uint64_t pol,
+                                                    uint8_t* out) {
+  const int fx = dir_dx(s.dir), fy = dir_dy(s.dir);
+  const auto cell = [&](int vi, int vj) -> uint32_t {
+    const int a = (kView - 1) - vj, b = vi - kView / 2;
+    const int wx = s.x + a * fx - b * fy, wy = s.y + a * fy + b * fx;
+    return ((unsigned)wx < (unsigned)W && (unsigned)wy < (unsigned)H) ? ld_cell(grid + wy * W + wx, pol) : CODE_WALL;
+  };
+  uint64_t transp = 0;
+#pragma unroll 1
+  for (int vj = 0; vj < kView; ++vj) {
+#pragma unroll
+    for (int vi = 0; vi < kView; ++vi)
+      if (!((M_OPAQUE >> (cell(vi, vj) & 0xf)) & 1u)) transp |= (uint64_t)1 << (vj * kView + vi);
+  }
+  const uint64_t vis = visibility(transp);
+#pragma unroll 1
+  for (int vi = 0; vi < kView; ++vi) {
+#pragma unroll
+    for (int vj = 0; vj < kView; ++vj) {
+      const bool agent_cell = (vi == kView / 2 && vj == kView - 1);
+      const uint32_t code = agent_cell ? (s.carry ? s.carry : CODE_EMPTY) : cell(vi, vj);
+      uint8_t t = 0, col = 0, stt = 0;
+      if ((vis >> (vj * kView + vi)) & 1) sym_of_code(code, t, col, stt);
+      uint8_t* o = out + (vi * kView + vj) * 3;
+      o[0] = t; o[1] = col; o[2] = stt;
+    }
+  }
+}
+
 // State phase, one env per lane, for the G envs e0 .. e0+G-1 (lanes >= G idle).  Must be called by a full warp.
 // Leaves kinds_s[lane][kKindStride] / sym_s[lane][147] filled for the envs whose bit is set in the returned mask.
 // SWAR = true: the observation is computed on window rows (obs_swar.cuh; needs W >= 7), else cell by cell.
@@ -74,8 +110,8 @@ __device__ __forceinline__ unsigned state_phase(const EnvParams& p, const Flags&
       const bool inb = (unsigned)fx < (unsigned)p.W && (unsigned)fy < (unsigned)p.H;
       const int fidx = fy * p.W + fx;
       const uint32_t fwd = inb ? ld_cell(grid + fidx, f.pol) : CODE_WALL;
-      const ActionDraw act = draw_action<STEP == 2>(p, f.n_actions, e);
-      commit_action<STEP == 2>(p, e, act);
+      const ActionDraw act = draw_action<step_draws(STEP)>(p, f.n_actions, e);
+      commit_action<step_draws(STEP)>(p, e, act);
       StepResult r = step_logic(s, act.action, f.n_actions, fwd, inb, fidx, p.max_steps);
       if (r.bad_action) atomicAdd(p.bad_actions, 1ull);
       if (r.write_idx >= 0 && f.mutable_grid) p.cells[(size_t)e * p.cell_stride + r.write_idx] = (uint8_t)r.write_code;
@@ -99,7 +135,11 @@ __device__ __forceinline__ unsigned state_phase(const EnvParams& p, const Flags&
       if (p.out_ep_length) p.out_ep_length[e] = done ? s.step_count : 0;
       if (p.out_stuck) p.out_stuck[e] = stuck ? 1 : 0;
       if (p.out_done) p.out_done[e] = done ? 1.f : 0.f;
-      record_first_episode<STEP == 2>(p, e, done, r.terminated && r.reward > 0.0, ep_ret, s.step_count);
+      record_first_episode<step_draws(STEP)>(p, e, done, r.terminated && r.reward > 0.0, ep_ret, s.step_count);
+      // the final image: after this lane's own grid write above, before the restart below replaces pose and grid
+      if constexpr (step_final(STEP)) {
+        if (done) store_final_row(s, grid, p.W, p.H, f.pol, p.final_sym + (size_t)e * kSymBytes);
+      }
       restart = done && f.auto_reset;
     }
   } else {
@@ -208,7 +248,8 @@ static bool use_swar(const EnvParams& p, const LaunchCtx& ctx, bool frame_kernel
   return ctx.observation_path == 2 || !frame_kernel;
 }
 
-// CTA-tile kernels (env_kernels_tile.cu): T = 16 or 8 envs per tile; `step` = 0 masked reset, 1 step, 2 policy step
+// CTA-tile kernels (env_kernels_tile.cu): T = 16 or 8 envs per tile; `step` = 0 masked reset, 1 step, 2 policy step,
+// 3 / 4 the same two recording final observations
 constexpr int kTileThreads = 128;
 constexpr int kTileCtasPerSm = 4;
 cudaError_t launch_tile_kernel(int T, int step, const EnvParams& p, const LaunchCtx& ctx, cudaStream_t stream);

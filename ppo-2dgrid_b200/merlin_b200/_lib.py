@@ -23,7 +23,8 @@ EXPORTS = (
     "merlin_set_kernel_choice", "merlin_set_observation_path", "merlin_env_step_kernel", "merlin_env_render", "merlin_env_render_f32", "merlin_env_full_obs", "merlin_gae",
     "merlin_pack_cell", "merlin_last_error", "merlin_version",
     "merlin_env_policy_step", "merlin_env_seed_sampler", "merlin_env_rearm", "merlin_env_set_kernel_choice",
-    "merlin_env_set_observation_path", "merlin_env_write_state",
+    "merlin_env_set_observation_path", "merlin_env_write_state", "merlin_env_step_final",
+    "merlin_env_policy_step_final", "merlin_env_final_step_kernel",
 )
 
 
@@ -75,6 +76,9 @@ def load():
     lib.merlin_env_reset.argtypes = [vp, vp, vp, vp, vp]
     lib.merlin_env_step.argtypes = [vp, vp, vp, vp, vp, vp, vp, C.POINTER(StepExtras), vp]
     lib.merlin_env_policy_step.argtypes = [vp, C.POINTER(PolicyIO), vp, vp, vp, vp, vp, C.POINTER(StepExtras), vp]
+    lib.merlin_env_step_final.argtypes = [vp, vp, vp, vp, vp, vp, vp, C.POINTER(StepExtras), vp, vp]
+    lib.merlin_env_policy_step_final.argtypes = [vp, C.POINTER(PolicyIO), vp, vp, vp, vp, vp, C.POINTER(StepExtras),
+                                                 vp, vp]
     lib.merlin_env_seed_sampler.argtypes = [vp, C.c_uint64]
     lib.merlin_env_rearm.argtypes = [vp, vp]
     lib.merlin_env_set_kernel_choice.argtypes = [vp, C.c_int]
@@ -98,6 +102,8 @@ def load():
     lib.merlin_env_render_f32.restype = C.c_int
     lib.merlin_env_step_kernel.argtypes = [vp, C.c_int]
     lib.merlin_env_step_kernel.restype = C.c_char_p
+    lib.merlin_env_final_step_kernel.argtypes = [vp, C.c_int]
+    lib.merlin_env_final_step_kernel.restype = C.c_char_p
     lib.merlin_gae.argtypes = [vp, vp, vp, vp, vp, vp, i32, i32, C.c_double, C.c_double, vp]
     lib.merlin_pack_cell.argtypes = [C.c_int, C.c_int, C.c_int]
     lib.merlin_pack_cell.restype = C.c_uint8
@@ -108,7 +114,7 @@ def load():
                  "merlin_env_set_cursors", "merlin_env_reset", "merlin_env_step", "merlin_env_state_ptrs",
                  "merlin_env_read_state", "merlin_env_bad_actions", "merlin_gae", "merlin_env_policy_step",
                  "merlin_env_seed_sampler", "merlin_env_rearm", "merlin_env_set_kernel_choice",
-                 "merlin_env_set_observation_path"):
+                 "merlin_env_set_observation_path", "merlin_env_step_final", "merlin_env_policy_step_final"):
         getattr(lib, name).restype = C.c_int
     _lib = lib
     if os.environ.get("MERLIN_OBSERVATION_PATH"):

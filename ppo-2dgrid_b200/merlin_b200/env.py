@@ -144,6 +144,7 @@ class BatchedMerlinEnv:
         self.done = torch.empty(N, dtype=torch.float32, device=dev)
         self._extras = _lib.StepExtras(self.episode_return.data_ptr(), self.episode_length.data_ptr(),
                                        self.stuck.data_ptr(), self.done.data_ptr())
+        self.final_obs_symbolic = None   # env-owned final-observation buffer (`step(..., final_obs=True)`)
         self.n_envs = self.num_envs
         # the in-kernel action sampler follows torch's seeding: key = hash(torch.initial_seed()) -- reproducible after
         # torch.manual_seed and different per rank when ranks seed differently; nothing is drawn from torch's generators.
@@ -249,12 +250,33 @@ class BatchedMerlinEnv:
                                               sym.data_ptr() if sym is not None else None, self._stream()))
         return obs, sym
 
-    def step(self, actions, out_obs=None, out_symbolic=None, out=None, frames=True):
+    def _final_buffer(self, final_obs):
+        """The u8[N, 7, 7, 3] tensor a step writes final observations into (`final_obs` of step / policy_step)."""
+        if final_obs is True:
+            if self.final_obs_symbolic is None:
+                if torch.cuda.is_current_stream_capturing():
+                    raise RuntimeError("final_obs=True allocates its buffer on first use: call it once before capture")
+                self.final_obs_symbolic = torch.empty((self.num_envs,) + SYM_SHAPE, dtype=torch.uint8,
+                                                      device=self.device)
+            return self.final_obs_symbolic
+        t = final_obs
+        if (not torch.is_tensor(t) or tuple(t.shape) != (self.num_envs,) + SYM_SHAPE or t.dtype != torch.uint8
+                or not t.is_contiguous() or t.device != self.device):
+            raise ValueError(f"final_obs must be True or a contiguous torch.uint8 tensor of shape "
+                             f"{(self.num_envs,) + SYM_SHAPE} on {self.device}")
+        return t
+
+    def step(self, actions, out_obs=None, out_symbolic=None, out=None, frames=True, final_obs=None):
         """actions: int64 CUDA tensor [N] (numpy/int lists are copied over).  Returns the gymnasium 5-tuple
         (obs u8[N,56,56,3], reward f32[N], terminated bool[N], truncated bool[N], info) with device tensors that
         are REUSED by the next call unless `out_obs` / `out_symbolic` point into caller storage (e.g. a rollout slot).
         `frames=False`: this call writes no RGB frames (obs is None; the symbolic-only kernel runs) -- for callers that
-        expand the symbolic image themselves (`render(..., dtype=torch.float32)` straight into the policy's input)."""
+        expand the symbolic image themselves (`render(..., dtype=torch.float32)` straight into the policy's input).
+        `final_obs`: a contiguous u8[N, 7, 7, 3] tensor on the env's device (e.g. a row of a [T, N, 7, 7, 3] rollout
+        tensor), or True for an env-owned one.  Row e then receives the symbolic observation of env e's terminal state
+        when its episode ends in this step -- before the auto-reset, as gymnasium's info["final_obs"] -- and is not
+        written otherwise; `info["final_obs_symbolic"]` is that tensor.  Everything else is exactly what the call
+        without it returns.  Frames of the terminal states: `render(info["final_obs_symbolic"], index=done_rows)`."""
         if not torch.is_tensor(actions):
             actions = torch.as_tensor(np.asarray(actions), dtype=torch.int64)
         if actions.device != self.device or actions.dtype != torch.int64 or not actions.is_contiguous():
@@ -264,12 +286,19 @@ class BatchedMerlinEnv:
         obs = (out_obs if out_obs is not None else self.obs) if frames else None
         sym = out_symbolic if out_symbolic is not None else self.obs_symbolic
         b = out if out is not None else self
-        _lib.check(self._lib.merlin_env_step(
-            self._h, actions.data_ptr(), obs.data_ptr() if obs is not None else None,
-            sym.data_ptr() if sym is not None else None, b.reward.data_ptr(), b.terminated.data_ptr(),
-            b.truncated.data_ptr(), C.byref(b._extras) if self.episode_stats else None, self._stream()))
+        args = (obs.data_ptr() if obs is not None else None, sym.data_ptr() if sym is not None else None,
+                b.reward.data_ptr(), b.terminated.data_ptr(), b.truncated.data_ptr(),
+                C.byref(b._extras) if self.episode_stats else None)
+        fin = None if final_obs is None else self._final_buffer(final_obs)
+        if fin is None:
+            _lib.check(self._lib.merlin_env_step(self._h, actions.data_ptr(), *args, self._stream()))
+        else:
+            _lib.check(self._lib.merlin_env_step_final(self._h, actions.data_ptr(), *args, fin.data_ptr(),
+                                                       self._stream()))
         info = {"episode_return": b.episode_return, "episode_length": b.episode_length, "stuck": b.stuck,
                 "done": b.done, "obs_symbolic": sym}
+        if fin is not None:
+            info["final_obs_symbolic"] = fin
         return obs, b.reward, b.terminated, b.truncated, info
 
     # ---- fused policy transition ------------------------------------------------------------------
@@ -321,20 +350,27 @@ class BatchedMerlinEnv:
         io._c = c
         return io
 
-    def policy_step(self, io, out_obs=None, out_symbolic=None, out=None, frames=True):
+    def policy_step(self, io, out_obs=None, out_symbolic=None, out=None, frames=True, final_obs=None):
         """One rollout transition in ONE launch: sample an action per env from `io.logits` (or argmax), store action /
         log-probability / value into `io`'s tensors, step every env and write the next observation.  Returns the same
         5-tuple as `step`; the action taken is `io.action`.  Replaces Categorical(logits).sample() + log_prob + env.step +
-        the rollout stores of src/ppo.py:70-86 and src/fomaml.py:65-84."""
+        the rollout stores of src/ppo.py:70-86 and src/fomaml.py:65-84.  `final_obs` as in `step`."""
         obs = (out_obs if out_obs is not None else self.obs) if frames else None
         sym = out_symbolic if out_symbolic is not None else self.obs_symbolic
         b = out if out is not None else self
-        _lib.check(self._lib.merlin_env_policy_step(
-            self._h, C.byref(io._c), obs.data_ptr() if obs is not None else None,
-            sym.data_ptr() if sym is not None else None, b.reward.data_ptr(), b.terminated.data_ptr(),
-            b.truncated.data_ptr(), C.byref(b._extras) if self.episode_stats else None, self._stream()))
+        args = (obs.data_ptr() if obs is not None else None, sym.data_ptr() if sym is not None else None,
+                b.reward.data_ptr(), b.terminated.data_ptr(), b.truncated.data_ptr(),
+                C.byref(b._extras) if self.episode_stats else None)
+        fin = None if final_obs is None else self._final_buffer(final_obs)
+        if fin is None:
+            _lib.check(self._lib.merlin_env_policy_step(self._h, C.byref(io._c), *args, self._stream()))
+        else:
+            _lib.check(self._lib.merlin_env_policy_step_final(self._h, C.byref(io._c), *args, fin.data_ptr(),
+                                                              self._stream()))
         info = {"episode_return": b.episode_return, "episode_length": b.episode_length, "stuck": b.stuck,
                 "done": b.done, "obs_symbolic": sym}
+        if fin is not None:
+            info["final_obs_symbolic"] = fin
         return obs, b.reward, b.terminated, b.truncated, info
 
     def set_kernel_choice(self, choice):
@@ -462,9 +498,10 @@ class BatchedMerlinEnv:
         _lib.check(self._lib.merlin_env_bad_actions(self._h, C.byref(n)))
         return n.value
 
-    def step_kernel(self):
-        """Name of the CUDA kernel `step` launches for this batch size / observation mode."""
-        return self._lib.merlin_env_step_kernel(self._h, 1 if self.want_rgb else 0).decode()
+    def step_kernel(self, final=False):
+        """Name of the CUDA kernel `step` launches for this batch size / observation mode (`final`: with final_obs)."""
+        fn = self._lib.merlin_env_final_step_kernel if final else self._lib.merlin_env_step_kernel
+        return fn(self._h, 1 if self.want_rgb else 0).decode()
 
     def launch_count(self):
         return int(self._lib.merlin_env_launch_count(self._h))

@@ -30,9 +30,16 @@ from .rollout_buffer import RolloutBuffer
 class PPO:
     def __init__(self, env, lr=3e-4, gamma=0.99, lam=0.95, clip_eps=0.2, update_epochs=10, batch_size=2048,
                  minibatch_size=256, vf_coef=0.5, ent_coef=0.01, device="cpu", use_cuda_graph=False,
-                 obs_storage="rgb", amp_dtype=None, minibatch_frames=torch.float32, carry_episodes=None):
+                 obs_storage="rgb", amp_dtype=None, minibatch_frames=torch.float32, carry_episodes=None,
+                 bootstrap_truncated=False):
         self.env = env
         self.batched = isinstance(env, BatchedMerlinEnv)
+        # bootstrap_truncated: an episode cut by the step limit is not a terminal state.  Its last reward gets
+        # gamma * V(final observation), the critic's value of the state the limit cut off (Stable-Baselines3's time-limit
+        # correction); GAE then treats the step as done as before.  False (default) = the reference: value 0.
+        if bootstrap_truncated and not self.batched:
+            raise ValueError("bootstrap_truncated needs a BatchedMerlinEnv (final observations come from its step kernel)")
+        self.bootstrap_truncated = bool(bootstrap_truncated)
         self.device = env.device if self.batched else torch.device(device)
         self.gamma, self.lam, self.clip_eps = gamma, lam, clip_eps
         self.update_epochs, self.batch_size, self.minibatch_size = update_epochs, batch_size, minibatch_size
@@ -92,11 +99,23 @@ class PPO:
             self._last_value = torch.zeros(N, dtype=torch.float32, device=self.device)
             # the step kernel writes reward / done / episode statistics of step t straight into row t of these tensors
             scratch = {k: torch.zeros(N, dtype=torch.bool, device=self.device) for k in ("terminated", "truncated", "stuck")}
+            if self.bootstrap_truncated:
+                # per-step flags, and the final observation of every episode that ends (u8[T, N, 7, 7, 3])
+                self._terminated = torch.zeros((T, N), dtype=torch.bool, device=self.device)
+                self._truncated = torch.zeros((T, N), dtype=torch.bool, device=self.device)
+                self._final_sym = torch.zeros((T, N, 7, 7, 3), dtype=torch.uint8, device=self.device)
+                self._boot_in = torch.zeros((min(self.minibatch_size, T * N), 14, 14, 48), dtype=torch.float32,
+                                            device=self.device)
 
             def row(x, t):
                 return x[t] if x.dim() == 2 else x[t:t + 1]
+            def flags(t):
+                if not self.bootstrap_truncated:
+                    return scratch
+                return dict(scratch, terminated=self._terminated[t], truncated=self._truncated[t])
             self._rows = [env.make_step_buffers(reward=row(self.buffer.rewards, t), done=row(self.buffer.dones, t),
-                                                episode_return=self._ep_ret[t], episode_length=self._ep_len[t], **scratch)
+                                                episode_return=self._ep_ret[t], episode_length=self._ep_len[t],
+                                                **flags(t))
                           for t in range(T)]
             # one fused transition per step: logits / value of step t -> action, log-probability, value rows of the buffer
             self._heads = torch.zeros((2, N, act_dim), dtype=torch.float32, device=self.device)
@@ -171,10 +190,11 @@ class PPO:
         for t in range(T):
             self._logits_value_into_heads(policy_input(t), lean)
             nxt = buf.obs_slot(t + 1) if t + 1 < T else last
+            fin = self._final_sym[t] if self.bootstrap_truncated else None
             if sym:  # symbolic storage: the symbolic-only kernel runs and writes NO frames
-                env.policy_step(self._ios[t], out_symbolic=nxt, out=self._rows[t], frames=False)
+                env.policy_step(self._ios[t], out_symbolic=nxt, out=self._rows[t], frames=False, final_obs=fin)
             else:
-                env.policy_step(self._ios[t], out_obs=nxt, out=self._rows[t])
+                env.policy_step(self._ios[t], out_obs=nxt, out=self._rows[t], final_obs=fin)
         self._logits_value_into_heads(policy_input(T), lean)
         self._last_value.copy_(self._heads[1, :, 0])
 
@@ -199,6 +219,8 @@ class PPO:
             self._graph[1].replay()
         else:
             self._rollout_body(fresh)
+        if self.bootstrap_truncated:
+            self._bootstrap_truncated()
         self._started = True
         ended = self._ep_len > 0  # one synchronisation per rollout, for the episode logs
         self.episode_returns.extend(self._ep_ret[ended].tolist())
@@ -206,6 +228,22 @@ class PPO:
         # episodes cut by the end of the rollout: continued next time (carry_episodes) or discarded by the next reset
         self.unfinished_episodes = int((self.buffer.dones[-1].reshape(-1) == 0).sum().item())
         return self._last_value
+
+    def _bootstrap_truncated(self):
+        """reward[t, e] += gamma * V(final observation of step t, env e) where step t truncated env e's episode and did
+        not terminate it.  Runs after the rollout (eager or replayed), before the parameters change: the frames of those
+        final observations are rendered into the policy's float32 input layout and valued in minibatch-sized chunks.
+        One host synchronisation (the number of truncated entries)."""
+        idx = (self._truncated & ~self._terminated).reshape(-1).nonzero().squeeze(1)
+        if idx.numel() == 0:
+            return
+        finals = self._final_sym.reshape(-1, 7, 7, 3)
+        rewards = self.buffer.rewards.reshape(-1)
+        for start in range(0, idx.numel(), self._boot_in.shape[0]):
+            rows = idx[start: start + self._boot_in.shape[0]]
+            x = self.env.render(finals, rows, out=self._boot_in[: rows.numel()], blocked=True, dtype=torch.float32)
+            value = self.ac(x)[1].float()
+            rewards.index_add_(0, rows, self.gamma * value)
 
     def _collect_single(self):
         state, _ = self.env.reset()

@@ -46,6 +46,8 @@ def main():
     ap.add_argument("--amp", choices=["none", "bf16"], default="none",
                     help="bf16 autocast for the policy evaluation in the update (reduced precision: not the headline setting)")
     ap.add_argument("--no-graph", action="store_true")
+    ap.add_argument("--bootstrap-truncated", action="store_true",
+                    help="add gamma * V(final observation) to the reward of steps cut by the episode step limit")
     ap.add_argument("--obs-storage", choices=["rgb", "symbolic"], default="symbolic",
                     help="rollout keeps 56x56x3 frames, or the 7x7x3 symbolic image rendered on read (64x smaller)")
     ap.add_argument("--mb-frames", choices=["f32", "u8"], default="f32",
@@ -100,7 +102,8 @@ def main():
                 batch_size=a.envs * a.horizon, minibatch_size=a.minibatch, vf_coef=0.5, ent_coef=a.ent_coef,
                 use_cuda_graph=not a.no_graph, obs_storage=a.obs_storage,
                 amp_dtype=torch.bfloat16 if a.amp == "bf16" else None,
-                minibatch_frames=torch.float32 if a.mb_frames == "f32" else torch.uint8)
+                minibatch_frames=torch.float32 if a.mb_frames == "f32" else torch.uint8,
+                bootstrap_truncated=a.bootstrap_truncated)
 
     def sync():
         if world > 1:
