@@ -107,11 +107,11 @@ __global__ void __launch_bounds__(kOrdThreads, kOrdCtas) env_kernel_ordered(cons
   __syncthreads();
 
   int g = 0;
-  if (lane == 0) g = (int)atomicAdd(&p.sched[0], 1u);
+  if (lane == 0) g = draw_ticket(p.sched);
   g = __shfl_sync(0xffffffffu, g, 0);
   while (g < n_groups) {
     int next = 0;
-    if (lane == 0) next = (int)atomicAdd(&p.sched[0], 1u);
+    if (lane == 0) next = draw_ticket(p.sched);
     const int e0 = g * kOrdG;
     const unsigned render_mask = state_phase<kOrdG, STEP, SWAR>(p, f, e0, lane, kinds_s, sym_s);
     if (f.want_sym && render_mask)
@@ -128,10 +128,7 @@ __global__ void __launch_bounds__(kOrdThreads, kOrdCtas) env_kernel_ordered(cons
     g = __shfl_sync(0xffffffffu, next, 0);
   }
   // every warp of the grid has drawn its last ticket once all of them have passed here: the last one rearms
-  if (lane == 0 && atomicAdd(&p.sched[1], 1u) == gridDim.x * (kOrdThreads / 32) - 1) {
-    p.sched[0] = 0;
-    p.sched[1] = 0;
-  }
+  if (lane == 0) rearm_tickets(p.sched, gridDim.x * (kOrdThreads / 32));
 }
 
 // ---------------------------------------------------------------------------------------------------
@@ -268,14 +265,15 @@ static cudaError_t launch_sized(const EnvParams& p, const LaunchCtx& ctx, cudaSt
       if (k.size == 16) return launch_group_kernel<16, STEP>(p, ctx, stream);
       if (k.size == 8) return launch_group_kernel<8, STEP>(p, ctx, stream);
       return launch_group_kernel<4, STEP>(p, ctx, stream);
-    case kChoiceTile: return launch_tile_kernel(k.size, STEP, p, ctx, stream);
-    case kChoiceTileTma: return launch_tile_tma_kernel(STEP, p, ctx, stream);
+    case kChoiceTile:
+      return k.size == 16 ? launch_tile_kernel<16, STEP>(p, ctx, stream) : launch_tile_kernel<8, STEP>(p, ctx, stream);
+    case kChoiceTileTma: return launch_tile_tma_kernel<STEP>(p, ctx, stream);
     case kChoiceSym: return launch_sym_kernel<STEP>(p, ctx, stream);
     case kChoiceOrdered: return launch_ordered_kernel<STEP>(p, ctx, stream);
     case kChoiceQuad:
-      if (STEP == 1 || STEP == 2) return launch_quad_kernel(STEP, p, ctx, stream);
-      return launch_warp_kernel(STEP, p, ctx, stream);   // the quad kernel only steps, without final observations
-    default: return launch_warp_kernel(STEP, p, ctx, stream);
+      if constexpr (STEP == 1 || STEP == 2) return launch_quad_kernel<STEP>(p, ctx, stream);
+      return launch_warp_kernel<STEP>(p, ctx, stream);   // the quad kernel only steps, without final observations
+    default: return launch_warp_kernel<STEP>(p, ctx, stream);
   }
 }
 

@@ -1,6 +1,9 @@
 // env_kernels_common.cuh -- device helpers and launch helpers shared by the kernel translation units
-// (env_kernels.cu: the large-batch step kernels and the launch policy; env_kernels_small.cu: the small-batch step
-// kernels; render_kernels.cu: frames from stored symbolic observations).
+// (env_kernels.cu: the group / ordered / symbolic-only step kernels and the launch policy; env_kernels_tile.cu: the
+// CTA-tile step kernels; env_kernels_small.cu: the small-batch step kernels; render_kernels.cu: frames from stored
+// symbolic observations).  Every per-env building block the six step-kernel mappings share -- the step outputs, the
+// restart, a window cell, the tile kind an observed cell shows, the work tickets -- is defined here once, and so are
+// the declarations of the launchers env_kernels.cu calls in the other translation units.
 #pragma once
 #include <cuda_runtime.h>
 #include <stdint.h>
@@ -123,6 +126,72 @@ __device__ __forceinline__ void record_first_episode(const EnvParams& p, int e, 
   p.rec_goal[e] = goal ? 1 : 0;
 }
 
+// Per-env outputs of a step: reward, the termination flags, and the optional episode-end / stuck / done rows.
+__device__ __forceinline__ void store_step_outputs(const EnvParams& p, int e, float rew, bool terminated, bool truncated,
+                                                   float ep_ret, int len, bool stuck) {
+  const bool done = terminated || truncated;
+  p.reward[e] = rew;
+  p.terminated[e] = terminated ? 1 : 0;
+  p.truncated[e] = truncated ? 1 : 0;
+  if (p.out_ep_return) p.out_ep_return[e] = done ? ep_ret : 0.f;
+  if (p.out_ep_length) p.out_ep_length[e] = done ? len : 0;
+  if (p.out_stuck) p.out_stuck[e] = stuck ? 1 : 0;
+  if (p.out_done) p.out_done[e] = done ? 1.f : 0.f;
+}
+
+// Restart: the pool slot an env loads -- its pending first layout, else the next (PPO) or the same (FOMAML) one.
+__device__ __forceinline__ int restart_layout(const EnvParams& p, bool advance, int layout) {
+  return layout < 0 ? ~layout
+                    : (advance ? (int)(((unsigned)layout + (unsigned)p.cursor_stride) % (unsigned)p.n_layouts) : layout);
+}
+// Restart pose from the pool's agent table, counters cleared.
+__device__ __forceinline__ void restart_state(const EnvParams& p, int layout, EnvState& s) {
+  const uint32_t a = p.pool_agent[layout];
+  s.x = a & 0xff; s.y = (a >> 8) & 0xff; s.dir = (a >> 16) & 3; s.carry = 0;
+  s.step_count = 0; s.stay = 0; s.last_x = s.x; s.last_y = s.y;
+}
+// Restart of a mutable grid: env e's private grid <- pool slot `layout`, by the 32 lanes of a warp.
+__device__ __forceinline__ void copy_pool_grid(const EnvParams& p, size_t e, int layout, int lane) {
+  const int4* from = reinterpret_cast<const int4*>(p.pool_cells + (size_t)layout * p.cell_stride);
+  int4* to = reinterpret_cast<int4*>(p.cells + e * p.cell_stride);
+  for (int i = lane; i < p.cell_stride / 16; i += 32) to[i] = from[i];
+}
+// Restart of the exploration bonus: env e's visited map <- only the cell (x, y), by the 32 lanes of a warp.
+__device__ __forceinline__ void reset_visited(const EnvParams& p, size_t e, int x, int y, int lane) {
+  const int cell = y * p.W + x;
+  for (int i = lane; i < p.vis_words; i += 32)
+    p.visited[e * p.vis_words + i] = (i == (cell >> 5)) ? (1u << (cell & 31)) : 0u;
+}
+
+// Code of grid cell (wx, wy); outside the grid it is a wall (Grid.slice).
+__device__ __forceinline__ uint32_t grid_cell(const uint8_t* grid, int W, int H, uint64_t pol, int wx, int wy) {
+  return ((unsigned)wx < (unsigned)W && (unsigned)wy < (unsigned)H) ? ld_cell(grid + wy * W + wx, pol) : CODE_WALL;
+}
+// Code of the cell `a` ahead of and `b` right of (x, y) for heading (fx, fy): window cell (vi, vj) is
+// a = 6 - vj, b = vi - 3.
+__device__ __forceinline__ uint32_t window_cell(const uint8_t* grid, int W, int H, uint64_t pol, int x, int y, int fx,
+                                                int fy, int a, int b) {
+  return grid_cell(grid, W, H, pol, x + a * fx - b * fy, y + a * fy + b * fx);
+}
+
+// One observed cell, `code` being what Grid.encode shows there -- at the agent cell what the agent carries
+// (carried_code).  shown_kind: the atlas slot of its tile -- the agent with its load at the agent cell, the unseen tile
+// where the cell is not visible, else the code.
+__device__ __forceinline__ uint32_t carried_code(uint32_t carry) { return carry ? carry : CODE_EMPTY; }
+__device__ __forceinline__ uint32_t shown_kind(uint32_t code, bool seen, bool agent_cell, uint32_t carry) {
+  return agent_cell ? agent_kind(carry) : (seen ? code : KIND_UNSEEN);
+}
+
+// In-order work tickets (tile, tile-TMA and ordered kernels): draw the next one; the last of `participants` to be done
+// drawing rearms the counters for the next launch (also under CUDA-graph replay).
+__device__ __forceinline__ int draw_ticket(unsigned* sched) { return (int)atomicAdd(&sched[0], 1u); }
+__device__ __forceinline__ void rearm_tickets(unsigned* sched, unsigned participants) {
+  if (atomicAdd(&sched[1], 1u) == participants - 1) {
+    sched[0] = 0;
+    sched[1] = 0;
+  }
+}
+
 // Stage the tile atlas: only the slots a frame of this handle's layout pool can show (5 of 128 for the MERLIN
 // scenarios: 960 B instead of 24 KB), at their usual offsets.  All threads of the CTA take part.
 __device__ __forceinline__ void stage_atlas(const EnvParams& p, uint8_t* atlas_s) {
@@ -203,9 +272,19 @@ static cudaError_t resident_ctas(const LaunchCtx& ctx, Kernel kernel, int thread
   return cudaSuccess;
 }
 
-// small-batch step kernels (env_kernels_small.cu); `step` = 0 masked reset, 1 step with given actions, 2 policy step,
-// 3 / 4 the same two recording final observations
-cudaError_t launch_warp_kernel(int step, const EnvParams& p, const LaunchCtx& ctx, cudaStream_t stream);
-cudaError_t launch_quad_kernel(int step, const EnvParams& p, const LaunchCtx& ctx, cudaStream_t stream);   // step 1 or 2
+// Launchers of the step kernels outside env_kernels.cu, instantiated in their own translation units for STEP = 0 masked
+// reset, 1 step with given actions, 2 policy step, 3 / 4 the same two recording final observations (the quad kernel:
+// 1 and 2 only).  CTA tiles (env_kernels_tile.cu): T = 16 or 8 envs per tile.
+constexpr int kTileThreads = 128;
+constexpr int kTileCtasPerSm = 4;
+template <int T, int STEP>
+cudaError_t launch_tile_kernel(const EnvParams& p, const LaunchCtx& ctx, cudaStream_t stream);
+template <int STEP>
+cudaError_t launch_tile_tma_kernel(const EnvParams& p, const LaunchCtx& ctx, cudaStream_t stream);
+// small-batch kernels (env_kernels_small.cu)
+template <int STEP>
+cudaError_t launch_warp_kernel(const EnvParams& p, const LaunchCtx& ctx, cudaStream_t stream);
+template <int STEP>
+cudaError_t launch_quad_kernel(const EnvParams& p, const LaunchCtx& ctx, cudaStream_t stream);
 
 }  // namespace merlin

@@ -157,15 +157,9 @@ __global__ void __launch_bounds__(kWarpKernelThreads, kWarpCtas) env_kernel_warp
       s.dir = a == A_LEFT ? (s.dir + 3) & 3 : (a == A_RIGHT ? (s.dir + 1) & 3 : s.dir);
       const uint8_t* grid = p.pool_cells + (size_t)s.layout * p.cell_stride;
       const int fx = dir_dx(s.dir), fy = dir_dy(s.dir);
-      uint32_t e0, e1 = CODE_WALL;
-      {
-        const int wx = s.x + (a0 + 1) * fx - b0 * fy, wy = s.y + (a0 + 1) * fy + b0 * fx;
-        e0 = ((unsigned)wx < (unsigned)p.W && (unsigned)wy < (unsigned)p.H) ? ld_cell(grid + wy * p.W + wx, f.pol) : CODE_WALL;
-      }
-      if (lane + 32 < kCells + kView) {
-        const int wx = s.x + (a1x + 1) * fx - b1x * fy, wy = s.y + (a1x + 1) * fy + b1x * fx;
-        e1 = ((unsigned)wx < (unsigned)p.W && (unsigned)wy < (unsigned)p.H) ? ld_cell(grid + wy * p.W + wx, f.pol) : CODE_WALL;
-      }
+      const uint32_t e0 = window_cell(grid, p.W, p.H, f.pol, s.x, s.y, fx, fy, a0 + 1, b0);
+      uint32_t e1 = CODE_WALL;
+      if (lane + 32 < kCells + kView) e1 = window_cell(grid, p.W, p.H, f.pol, s.x, s.y, fx, fy, a1x + 1, b1x);
       const uint32_t ft = __shfl_sync(0xffffffffu, e1, 45 - 32) & 0xf;   // the cell ahead: ext row 6, column 3
       s.step_count += 1;
       const bool fwd_act = a == A_FORWARD;
@@ -182,13 +176,7 @@ __global__ void __launch_bounds__(kWarpKernelThreads, kWarpCtas) env_kernel_warp
         commit_action<step_draws(STEP)>(p, e, act);
         record_first_episode<step_draws(STEP)>(p, e, done, goal && rew > 0.f, ep_ret, s.step_count);
         if (bad) atomicAdd(p.bad_actions, 1ull);
-        p.reward[e] = rew;
-        p.terminated[e] = terminated ? 1 : 0;
-        p.truncated[e] = truncated ? 1 : 0;
-        if (p.out_ep_return) p.out_ep_return[e] = done ? ep_ret : 0.f;
-        if (p.out_ep_length) p.out_ep_length[e] = done ? s.step_count : 0;
-        if (p.out_stuck) p.out_stuck[e] = 0;
-        if (p.out_done) p.out_done[e] = done ? 1.f : 0.f;
+        store_step_outputs(p, e, rew, terminated, truncated, ep_ret, s.step_count, false);
       }
       restart = done && f.auto_reset;
       const int rot = (lane + kView) & 31;
@@ -228,28 +216,16 @@ __global__ void __launch_bounds__(kWarpKernelThreads, kWarpCtas) env_kernel_warp
         if (r.bad_action) atomicAdd(p.bad_actions, 1ull);
         if (r.write_idx >= 0 && f.mutable_grid) p.cells[(size_t)e * p.cell_stride + r.write_idx] = (uint8_t)r.write_code;
         if (f.explore_on && vword != vword_in) *vptr = vword;
-        p.reward[e] = rew;
-        p.terminated[e] = r.terminated ? 1 : 0;
-        p.truncated[e] = r.truncated ? 1 : 0;
-        if (p.out_ep_return) p.out_ep_return[e] = done ? ep_ret : 0.f;
-        if (p.out_ep_length) p.out_ep_length[e] = done ? s.step_count : 0;
-        if (p.out_stuck) p.out_stuck[e] = stuck ? 1 : 0;
-        if (p.out_done) p.out_done[e] = done ? 1.f : 0.f;
+        store_step_outputs(p, e, rew, r.terminated, r.truncated, ep_ret, s.step_count, stuck);
       }
       // final image (warp-uniform): the window after lane 0's grid write above, before the restart copy below
       if constexpr (step_final(STEP)) {
         if (done) {
           __syncwarp();
           const int fx = dir_dx(s.dir), fy = dir_dy(s.dir);
-          uint32_t w0, w1 = CODE_WALL;
-          {
-            const int wx = s.x + a0 * fx - b0 * fy, wy = s.y + a0 * fy + b0 * fx;
-            w0 = ((unsigned)wx < (unsigned)p.W && (unsigned)wy < (unsigned)p.H) ? ld_cell(grid + wy * p.W + wx, f.pol) : CODE_WALL;
-          }
-          if (c1 < kCells) {
-            const int wx = s.x + a1 * fx - b1 * fy, wy = s.y + a1 * fy + b1 * fx;
-            w1 = ((unsigned)wx < (unsigned)p.W && (unsigned)wy < (unsigned)p.H) ? ld_cell(grid + wy * p.W + wx, f.pol) : CODE_WALL;
-          }
+          const uint32_t w0 = window_cell(grid, p.W, p.H, f.pol, s.x, s.y, fx, fy, a0, b0);
+          uint32_t w1 = CODE_WALL;
+          if (c1 < kCells) w1 = window_cell(grid, p.W, p.H, f.pol, s.x, s.y, fx, fy, a1, b1);
           warp_store_final(w0, w1, lane, s.carry, p.final_sym + (size_t)e * kSymBytes);
         }
       }
@@ -260,24 +236,17 @@ __global__ void __launch_bounds__(kWarpKernelThreads, kWarpCtas) env_kernel_warp
     }
 
     if (restart) {  // warp-uniform
-      const int load_cur = s.layout < 0 ? ~s.layout
-                                        : (f.advance ? (int)(((unsigned)s.layout + (unsigned)p.cursor_stride) % (unsigned)p.n_layouts) : s.layout);
-      const uint32_t a = p.pool_agent[load_cur];
-      s.x = a & 0xff; s.y = (a >> 8) & 0xff; s.dir = (a >> 16) & 3; s.carry = 0;
-      s.step_count = 0; s.stay = 0; s.last_x = s.x; s.last_y = s.y;
+      const int load_cur = restart_layout(p, f.advance, s.layout);
+      restart_state(p, load_cur, s);
       ep_ret = 0.f;
       s.layout = load_cur;
       if (!LEAN && f.mutable_grid) {
         __syncwarp();
-        const int4* from = reinterpret_cast<const int4*>(p.pool_cells + (size_t)load_cur * p.cell_stride);
-        int4* to = reinterpret_cast<int4*>(p.cells + (size_t)e * p.cell_stride);
-        for (int i = lane; i < p.cell_stride / 16; i += 32) to[i] = from[i];
+        copy_pool_grid(p, (size_t)e, load_cur, lane);
       }
       if (!LEAN && f.explore_on) {
         __syncwarp();
-        const int cell = s.y * p.W + s.x;
-        for (int i = lane; i < p.vis_words; i += 32)
-          p.visited[(size_t)e * p.vis_words + i] = (i == (cell >> 5)) ? (1u << (cell & 31)) : 0u;
+        reset_visited(p, (size_t)e, s.x, s.y, lane);
       }
     }
     if (lane == 0 && (STEP || restart)) {
@@ -295,15 +264,11 @@ __global__ void __launch_bounds__(kWarpKernelThreads, kWarpCtas) env_kernel_warp
                                            : p.pool_cells + (size_t)s.layout * p.cell_stride;
       const int fx = dir_dx(s.dir), fy = dir_dy(s.dir);
       const int rx = -fy, ry = fx;
+      // window_cell's arithmetic spelled with the right vector (rx, ry): this form keeps the lean STEP = 4 instances at
+      // their instruction count (through window_cell they take 8 more)
       code1 = CODE_WALL;
-      {
-        const int wx = s.x + a0 * fx + b0 * rx, wy = s.y + a0 * fy + b0 * ry;
-        code0 = ((unsigned)wx < (unsigned)p.W && (unsigned)wy < (unsigned)p.H) ? ld_cell(grid + wy * p.W + wx, f.pol) : CODE_WALL;
-      }
-      if (c1 < kCells) {
-        const int wx = s.x + a1 * fx + b1 * rx, wy = s.y + a1 * fy + b1 * ry;
-        code1 = ((unsigned)wx < (unsigned)p.W && (unsigned)wy < (unsigned)p.H) ? ld_cell(grid + wy * p.W + wx, f.pol) : CODE_WALL;
-      }
+      code0 = grid_cell(grid, p.W, p.H, f.pol, s.x + a0 * fx + b0 * rx, s.y + a0 * fy + b0 * ry);
+      if (c1 < kCells) code1 = grid_cell(grid, p.W, p.H, f.pol, s.x + a1 * fx + b1 * rx, s.y + a1 * fy + b1 * ry);
     }
     const unsigned t0 = __ballot_sync(0xffffffffu, !((M_OPAQUE >> (code0 & 0xf)) & 1u));
     const unsigned t1 = __ballot_sync(0xffffffffu, c1 < kCells && !((M_OPAQUE >> (code1 & 0xf)) & 1u));
@@ -317,7 +282,7 @@ __global__ void __launch_bounds__(kWarpKernelThreads, kWarpCtas) env_kernel_warp
       uint32_t code = h ? code1 : code0;
       const bool seen = (vis >> c) & 1;
       const bool agent_cell = (vi == kView / 2 && vj == kView - 1);
-      if (agent_cell) code = s.carry ? s.carry : CODE_EMPTY;
+      if (agent_cell) code = carried_code(s.carry);
       const int k = vi * kView + vj;
       kq[k] = (uint16_t)((agent_cell ? agent_kind(s.carry) : (seen ? code : KIND_UNSEEN)) * kTileBytes);
       if (f.want_sym) {
@@ -378,7 +343,7 @@ __device__ __forceinline__ void load_ext_row(const EnvParams& p, const uint8_t* 
   uint32_t c[kView];
 #pragma unroll
   for (int vi = 0; vi < kView; ++vi) {
-    c[vi] = ((unsigned)wx < (unsigned)p.W && (unsigned)wy < (unsigned)p.H) ? ld_cell(grid + wy * p.W + wx, pol) : CODE_WALL;
+    c[vi] = grid_cell(grid, p.W, p.H, pol, wx, wy);
     wx -= fy; wy += fx;
   }
   codes = 0; transp = 0;
@@ -485,17 +450,10 @@ __global__ void __launch_bounds__(kWarpKernelThreads, kQuadCtas) env_kernel_quad
       commit_action<step_draws(STEP)>(p, e, act);
       record_first_episode<step_draws(STEP)>(p, e, done, goal && rew > 0.f, ep_ret, step_count);
       if (bad) atomicAdd(p.bad_actions, 1ull);
-      p.reward[e] = rew;
-      p.terminated[e] = terminated ? 1 : 0;
-      p.truncated[e] = truncated ? 1 : 0;
-      if (p.out_ep_return) p.out_ep_return[e] = done ? ep_ret : 0.f;
-      if (p.out_ep_length) p.out_ep_length[e] = done ? step_count : 0;
-      if (p.out_stuck) p.out_stuck[e] = 0;
-      if (p.out_done) p.out_done[e] = done ? 1.f : 0.f;
+      store_step_outputs(p, e, rew, terminated, truncated, ep_ret, step_count, false);
     }
     if (done && auto_reset) {   // uniform within the group
-      const int load_cur = layout < 0 ? ~layout
-                                      : (advance ? (int)(((unsigned)layout + (unsigned)p.cursor_stride) % (unsigned)p.n_layouts) : layout);
+      const int load_cur = restart_layout(p, advance, layout);
       const uint32_t pa = p.pool_agent[load_cur];
       x = pa & 0xff; y = (pa >> 8) & 0xff; dir = (pa >> 16) & 3; carry = 0;
       step_count = 0; sw = (x << 16) | (int)((uint32_t)y << 24);
@@ -530,8 +488,8 @@ __global__ void __launch_bounds__(kWarpKernelThreads, kQuadCtas) env_kernel_quad
         const bool seen = (visrow >> vi) & 1u;
         const bool agent_cell = vi == kView / 2 && r == kView - 1;
         uint32_t code = (uint32_t)(w >> (8 * vi)) & 0xff;
-        if (agent_cell) code = carry ? carry : CODE_EMPTY;
-        kd[vi * kView] = (uint16_t)((agent_cell ? agent_kind(carry) : (seen ? code : KIND_UNSEEN)) * kTileBytes);
+        if (agent_cell) code = carried_code(carry);
+        kd[vi * kView] = (uint16_t)(shown_kind(code, seen, agent_cell, carry) * kTileBytes);
         if (so) {   // Grid.encode of the cell, (0, 0, 0) when not visible: bytes (vi * 7 + vj) * 3 ..
           uint8_t t = 0, col = 0, stt = 0;
           if (seen) sym_of_code(code, t, col, stt);
@@ -612,7 +570,7 @@ static cudaError_t launch_warp_kernel_impl(const EnvParams& p, const LaunchCtx& 
 // other warps' stores) the lean form's 56-cell region and shuffles cost 1.5 % (27.5 vs 27.0 us).
 constexpr int kWarpLeanMaxEnvs = 12288;
 template <int STEP>
-static cudaError_t launch_warp_kernel_step(const EnvParams& p, const LaunchCtx& ctx, cudaStream_t stream) {
+cudaError_t launch_warp_kernel(const EnvParams& p, const LaunchCtx& ctx, cudaStream_t stream) {
   if constexpr (STEP != 0) {
     if (p.N <= kWarpLeanMaxEnvs && lean_config(p.flags)) return launch_warp_kernel_impl<STEP, true>(p, ctx, stream);
   }
@@ -624,7 +582,7 @@ static cudaError_t launch_warp_kernel_step(const EnvParams& p, const LaunchCtx& 
 // resident behind it, and a step then takes twice as long (4096 envs = 147 CTAs: 16 us instead of 9).
 constexpr int kQuadPdlMinEnvs = 16384;
 template <int STEP>
-static cudaError_t launch_quad_kernel_step(const EnvParams& p, const LaunchCtx& ctx, cudaStream_t stream) {
+cudaError_t launch_quad_kernel(const EnvParams& p, const LaunchCtx& ctx, cudaStream_t stream) {
   const size_t smem = kAtlasBytes + (kWarpKernelThreads / 32) * kQuadKindBytes;
   const bool pdl = p.N >= kQuadPdlMinEnvs;
   const auto kernel = pdl ? env_kernel_quad<STEP, true> : env_kernel_quad<STEP, false>;
@@ -635,15 +593,12 @@ static cudaError_t launch_quad_kernel_step(const EnvParams& p, const LaunchCtx& 
   return launch_maybe_pdl(kernel, pdl, grid, threads, smem, stream, p);
 }
 
-cudaError_t launch_warp_kernel(int step, const EnvParams& p, const LaunchCtx& ctx, cudaStream_t stream) {
-  if (step == 0) return launch_warp_kernel_step<0>(p, ctx, stream);
-  if (step == 1) return launch_warp_kernel_step<1>(p, ctx, stream);
-  if (step == 3) return launch_warp_kernel_step<3>(p, ctx, stream);
-  if (step == 4) return launch_warp_kernel_step<4>(p, ctx, stream);
-  return launch_warp_kernel_step<2>(p, ctx, stream);
-}
-cudaError_t launch_quad_kernel(int step, const EnvParams& p, const LaunchCtx& ctx, cudaStream_t stream) {
-  return step == 2 ? launch_quad_kernel_step<2>(p, ctx, stream) : launch_quad_kernel_step<1>(p, ctx, stream);
-}
+template cudaError_t launch_warp_kernel<0>(const EnvParams&, const LaunchCtx&, cudaStream_t);
+template cudaError_t launch_warp_kernel<1>(const EnvParams&, const LaunchCtx&, cudaStream_t);
+template cudaError_t launch_warp_kernel<2>(const EnvParams&, const LaunchCtx&, cudaStream_t);
+template cudaError_t launch_warp_kernel<3>(const EnvParams&, const LaunchCtx&, cudaStream_t);
+template cudaError_t launch_warp_kernel<4>(const EnvParams&, const LaunchCtx&, cudaStream_t);
+template cudaError_t launch_quad_kernel<1>(const EnvParams&, const LaunchCtx&, cudaStream_t);
+template cudaError_t launch_quad_kernel<2>(const EnvParams&, const LaunchCtx&, cudaStream_t);
 
 }  // namespace merlin

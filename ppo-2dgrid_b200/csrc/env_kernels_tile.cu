@@ -53,7 +53,7 @@ __global__ void __launch_bounds__(kTileThreads, kTileCtasPerSm) env_kernel_tile(
   // `tile += gridDim.x` assignment, whose CTAs drift apart).  Thread 32 draws the next ticket while warp 0 runs the
   // state phase; the last CTA to finish rearms the counters for the next launch (also under CUDA-graph replay).
   __shared__ int s_next;
-  if (threadIdx.x == 0) s_next = (int)atomicAdd(&p.sched[0], 1u);
+  if (threadIdx.x == 0) s_next = draw_ticket(p.sched);
   __syncthreads();
   int tile = s_next;
   while (tile < n_tiles) {
@@ -62,7 +62,7 @@ __global__ void __launch_bounds__(kTileThreads, kTileCtasPerSm) env_kernel_tile(
       const unsigned m = state_phase<T, STEP, SWAR>(p, f, e0, lane, kinds_s, sym_s);
       if (lane == 0) *mask_s = m;
     } else if (threadIdx.x == 32) {
-      s_next = (int)atomicAdd(&p.sched[0], 1u);
+      s_next = draw_ticket(p.sched);
     }
     __syncthreads();  // kinds / sym / mask of this tile, the next ticket (and, first time round, the atlas) are in smem
     const unsigned render_mask = *mask_s;
@@ -77,10 +77,7 @@ __global__ void __launch_bounds__(kTileThreads, kTileCtasPerSm) env_kernel_tile(
     __syncthreads();  // the tile buffers and the ticket slot are rewritten in the next round
     tile = next;
   }
-  if (threadIdx.x == 0 && atomicAdd(&p.sched[1], 1u) == gridDim.x - 1) {
-    p.sched[0] = 0;  // every CTA has drawn its last ticket: safe to rearm
-    p.sched[1] = 0;
-  }
+  if (threadIdx.x == 0) rearm_tickets(p.sched, gridDim.x);   // every CTA has drawn its last ticket
 }
 
 // ---------------------------------------------------------------------------------------------------
@@ -150,7 +147,7 @@ __global__ void __launch_bounds__(kTmaThreads, kTmaCtas) env_kernel_tile_tma(con
   }
   int buf = 0;
   __shared__ int s_next;
-  if (threadIdx.x == 0) s_next = (int)atomicAdd(&p.sched[0], 1u);
+  if (threadIdx.x == 0) s_next = draw_ticket(p.sched);
   __syncthreads();
   int tile = s_next;
   while (tile < n_tiles) {
@@ -159,7 +156,7 @@ __global__ void __launch_bounds__(kTmaThreads, kTmaCtas) env_kernel_tile_tma(con
       const unsigned m = state_phase<kTmaT, STEP>(p, f, e0, lane, kinds_s, sym_s);
       if (lane == 0) *mask_s = m;
     } else if (threadIdx.x == 32) {
-      s_next = (int)atomicAdd(&p.sched[0], 1u);
+      s_next = draw_ticket(p.sched);
     }
     __syncthreads();
     const unsigned render_mask = *mask_s;
@@ -183,10 +180,7 @@ __global__ void __launch_bounds__(kTmaThreads, kTmaCtas) env_kernel_tile_tma(con
     tile = next;
   }
   if (lane == 0) bulk_wait_read<0>();   // shared memory must outlive the engine's reads
-  if (threadIdx.x == 0 && atomicAdd(&p.sched[1], 1u) == gridDim.x - 1) {
-    p.sched[0] = 0;
-    p.sched[1] = 0;
-  }
+  if (threadIdx.x == 0) rearm_tickets(p.sched, gridDim.x);
 }
 
 template <int T, int STEP, bool SWAR>
@@ -201,13 +195,13 @@ static cudaError_t launch_tile_kernel_impl(const EnvParams& p, const LaunchCtx& 
   return cudaGetLastError();
 }
 template <int T, int STEP>
-static cudaError_t launch_tile_kernel_step(const EnvParams& p, const LaunchCtx& ctx, cudaStream_t stream) {
+cudaError_t launch_tile_kernel(const EnvParams& p, const LaunchCtx& ctx, cudaStream_t stream) {
   return use_swar(p, ctx, true) ? launch_tile_kernel_impl<T, STEP, true>(p, ctx, stream)
                                 : launch_tile_kernel_impl<T, STEP, false>(p, ctx, stream);
 }
 
 template <int STEP>
-static cudaError_t launch_tile_tma_kernel_step(const EnvParams& p, const LaunchCtx& ctx, cudaStream_t stream) {
+cudaError_t launch_tile_tma_kernel(const EnvParams& p, const LaunchCtx& ctx, cudaStream_t stream) {
   const int n_tiles = (p.N + kTmaT - 1) / kTmaT;
   int ctas;
   if (cudaError_t err = resident_ctas(ctx, env_kernel_tile_tma<STEP>, kTmaThreads, kTmaSmemBytes, ctas, kTmaCtas))
@@ -217,26 +211,15 @@ static cudaError_t launch_tile_tma_kernel_step(const EnvParams& p, const LaunchC
   return cudaGetLastError();
 }
 
-cudaError_t launch_tile_kernel(int T, int step, const EnvParams& p, const LaunchCtx& ctx, cudaStream_t stream) {
-  if (T == 16) {
-    if (step == 0) return launch_tile_kernel_step<16, 0>(p, ctx, stream);
-    if (step == 1) return launch_tile_kernel_step<16, 1>(p, ctx, stream);
-    if (step == 3) return launch_tile_kernel_step<16, 3>(p, ctx, stream);
-    if (step == 4) return launch_tile_kernel_step<16, 4>(p, ctx, stream);
-    return launch_tile_kernel_step<16, 2>(p, ctx, stream);
-  }
-  if (step == 0) return launch_tile_kernel_step<8, 0>(p, ctx, stream);
-  if (step == 1) return launch_tile_kernel_step<8, 1>(p, ctx, stream);
-  if (step == 3) return launch_tile_kernel_step<8, 3>(p, ctx, stream);
-  if (step == 4) return launch_tile_kernel_step<8, 4>(p, ctx, stream);
-  return launch_tile_kernel_step<8, 2>(p, ctx, stream);
-}
-cudaError_t launch_tile_tma_kernel(int step, const EnvParams& p, const LaunchCtx& ctx, cudaStream_t stream) {
-  if (step == 0) return launch_tile_tma_kernel_step<0>(p, ctx, stream);
-  if (step == 1) return launch_tile_tma_kernel_step<1>(p, ctx, stream);
-  if (step == 3) return launch_tile_tma_kernel_step<3>(p, ctx, stream);
-  if (step == 4) return launch_tile_tma_kernel_step<4>(p, ctx, stream);
-  return launch_tile_tma_kernel_step<2>(p, ctx, stream);
-}
+#define MERLIN_TILE_LAUNCHERS(STEP)                                                                      \
+  template cudaError_t launch_tile_kernel<16, STEP>(const EnvParams&, const LaunchCtx&, cudaStream_t);   \
+  template cudaError_t launch_tile_kernel<8, STEP>(const EnvParams&, const LaunchCtx&, cudaStream_t);    \
+  template cudaError_t launch_tile_tma_kernel<STEP>(const EnvParams&, const LaunchCtx&, cudaStream_t);
+MERLIN_TILE_LAUNCHERS(0)
+MERLIN_TILE_LAUNCHERS(1)
+MERLIN_TILE_LAUNCHERS(2)
+MERLIN_TILE_LAUNCHERS(3)
+MERLIN_TILE_LAUNCHERS(4)
+#undef MERLIN_TILE_LAUNCHERS
 
 }  // namespace merlin

@@ -59,9 +59,7 @@ static __device__ __noinline__ void store_final_row(const EnvState& s, const uin
                                                     uint8_t* out) {
   const int fx = dir_dx(s.dir), fy = dir_dy(s.dir);
   const auto cell = [&](int vi, int vj) -> uint32_t {
-    const int a = (kView - 1) - vj, b = vi - kView / 2;
-    const int wx = s.x + a * fx - b * fy, wy = s.y + a * fy + b * fx;
-    return ((unsigned)wx < (unsigned)W && (unsigned)wy < (unsigned)H) ? ld_cell(grid + wy * W + wx, pol) : CODE_WALL;
+    return window_cell(grid, W, H, pol, s.x, s.y, fx, fy, (kView - 1) - vj, vi - kView / 2);
   };
   uint64_t transp = 0;
 #pragma unroll 1
@@ -76,7 +74,7 @@ static __device__ __noinline__ void store_final_row(const EnvState& s, const uin
 #pragma unroll
     for (int vj = 0; vj < kView; ++vj) {
       const bool agent_cell = (vi == kView / 2 && vj == kView - 1);
-      const uint32_t code = agent_cell ? (s.carry ? s.carry : CODE_EMPTY) : cell(vi, vj);
+      const uint32_t code = agent_cell ? carried_code(s.carry) : cell(vi, vj);
       uint8_t t = 0, col = 0, stt = 0;
       if ((vis >> (vj * kView + vi)) & 1) sym_of_code(code, t, col, stt);
       uint8_t* o = out + (vi * kView + vj) * 3;
@@ -128,13 +126,7 @@ __device__ __forceinline__ unsigned state_phase(const EnvParams& p, const Flags&
       const float rew = (float)rew_d;
       ep_ret += rew;
       const bool done = r.terminated || r.truncated;
-      p.reward[e] = rew;
-      p.terminated[e] = r.terminated ? 1 : 0;
-      p.truncated[e] = r.truncated ? 1 : 0;
-      if (p.out_ep_return) p.out_ep_return[e] = done ? ep_ret : 0.f;
-      if (p.out_ep_length) p.out_ep_length[e] = done ? s.step_count : 0;
-      if (p.out_stuck) p.out_stuck[e] = stuck ? 1 : 0;
-      if (p.out_done) p.out_done[e] = done ? 1.f : 0.f;
+      store_step_outputs(p, e, rew, r.terminated, r.truncated, ep_ret, s.step_count, stuck);
       record_first_episode<step_draws(STEP)>(p, e, done, r.terminated && r.reward > 0.0, ep_ret, s.step_count);
       // the final image: after this lane's own grid write above, before the restart below replaces pose and grid
       if constexpr (step_final(STEP)) {
@@ -151,13 +143,9 @@ __device__ __forceinline__ unsigned state_phase(const EnvParams& p, const Flags&
   // re-initialised by the whole warp with coalesced copies
   const unsigned restart_mask = __ballot_sync(0xffffffffu, restart);
   if (restart_mask) {
-    // pool index this env loads: pending first layout, else the next (PPO) or the same (FOMAML) one
-    const int load_cur = s.layout < 0 ? ~s.layout
-                                      : (f.advance ? (int)(((unsigned)s.layout + (unsigned)p.cursor_stride) % (unsigned)p.n_layouts) : s.layout);
+    const int load_cur = restart_layout(p, f.advance, s.layout);
     if (restart) {
-      const uint32_t a = p.pool_agent[load_cur];
-      s.x = a & 0xff; s.y = (a >> 8) & 0xff; s.dir = (a >> 16) & 3; s.carry = 0;
-      s.step_count = 0; s.stay = 0; s.last_x = s.x; s.last_y = s.y;
+      restart_state(p, load_cur, s);
       ep_ret = 0.f;
     }
     if (f.mutable_grid || f.explore_on) {
@@ -168,16 +156,8 @@ __device__ __forceinline__ unsigned state_phase(const EnvParams& p, const Flags&
         const int cur = __shfl_sync(0xffffffffu, load_cur, src);
         const int sx = __shfl_sync(0xffffffffu, s.x, src), sy = __shfl_sync(0xffffffffu, s.y, src);
         const size_t ee = (size_t)(e0 + src);
-        if (f.mutable_grid) {
-          const int4* from = reinterpret_cast<const int4*>(p.pool_cells + (size_t)cur * p.cell_stride);
-          int4* to = reinterpret_cast<int4*>(p.cells + ee * p.cell_stride);
-          for (int i = lane; i < p.cell_stride / 16; i += 32) to[i] = from[i];
-        }
-        if (f.explore_on) {
-          const int cell = sy * p.W + sx;
-          for (int i = lane; i < p.vis_words; i += 32)
-            p.visited[ee * p.vis_words + i] = (i == (cell >> 5)) ? (1u << (cell & 31)) : 0u;
-        }
+        if (f.mutable_grid) copy_pool_grid(p, ee, cur, lane);
+        if (f.explore_on) reset_visited(p, ee, sx, sy, lane);
       }
       __syncwarp();
     }
@@ -220,8 +200,8 @@ __device__ __forceinline__ unsigned state_phase(const EnvParams& p, const Flags&
           const bool seen = (vis >> (vj * kView + vi)) & 1;
           uint32_t code = kind[c];
           const bool agent_cell = (vi == kView / 2 && vj == kView - 1);
-          if (agent_cell) code = s.carry ? s.carry : CODE_EMPTY;
-          kind[c] = (uint8_t)(agent_cell ? agent_kind(s.carry) : (seen ? code : KIND_UNSEEN));
+          if (agent_cell) code = carried_code(s.carry);
+          kind[c] = (uint8_t)shown_kind(code, seen, agent_cell, s.carry);
           if (f.want_sym) {
             uint8_t t = 0, col = 0, stt = 0;
             if (seen) sym_of_code(code, t, col, stt);
@@ -247,12 +227,5 @@ static bool use_swar(const EnvParams& p, const LaunchCtx& ctx, bool frame_kernel
   if (p.W < kView || ctx.observation_path == 1) return false;
   return ctx.observation_path == 2 || !frame_kernel;
 }
-
-// CTA-tile kernels (env_kernels_tile.cu): T = 16 or 8 envs per tile; `step` = 0 masked reset, 1 step, 2 policy step,
-// 3 / 4 the same two recording final observations
-constexpr int kTileThreads = 128;
-constexpr int kTileCtasPerSm = 4;
-cudaError_t launch_tile_kernel(int T, int step, const EnvParams& p, const LaunchCtx& ctx, cudaStream_t stream);
-cudaError_t launch_tile_tma_kernel(int step, const EnvParams& p, const LaunchCtx& ctx, cudaStream_t stream);
 
 }  // namespace merlin
